@@ -174,6 +174,33 @@ def algorithmic_bytes_per_env_step(nq, nv, nj, kbar):
     return 4.0 * (2 * nq + 3 * nv + 2 * nj + 1 + 12.0 * kbar)
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def write_outputs(path, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array, every array one row per environment (all ranks, rank order):
+      obs      observation rows of the last timed step of the device-resident arm (the headline value's path)
+      gc, gv   generalized coordinates / velocities right after that step
+      obs_e2e  observation rows of the last timed step of the host-buffer (e2e) arm
+    The workload is seeded, so the same arguments give the same inputs on every run and two builds can be compared file by file.
+    Above DUMP_MAX_BYTES in all, a fixed, seeded sample of environments is kept: the same rows of every array, their indices in
+    env_index.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.asarray(a, np.float64 if a.dtype == np.float64 else np.float32) for k, a in arrays.items()}
+    rows = {a.shape[0] for a in arrays.values()}
+    assert len(rows) == 1, {k: a.shape for k, a in arrays.items()}
+    rows = rows.pop()
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    budget = DUMP_MAX_BYTES - 4096                    # headroom for the .npy headers
+    if rows * row_bytes > budget:
+        keep = budget // (row_bytes + 8)
+        idx = np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 # ------------------------------------------------------------------ CPU arm --------------------------
 class CpuSim:
     """the oracle port driving one Workload (a restatement of World::integrate(), NOT RaiSim's binary): OpenMP over
@@ -386,6 +413,7 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-side-results", action="store_true")
     ap.add_argument("--nccl-gather", action="store_true", help="N > 1: NCCL all-gather after the step instead of the fused peer-memory gather, for comparison")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy (see write_outputs)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -431,30 +459,33 @@ def main():
     def timed(host_io, steps, step0):
         # one event pair per step around the whole step (ms_per_step); a second pair around the launch alone only where the step
         # holds more than the launch (the NCCL arm's all-gather: with the fused peer gather the arrival wait is part of the launch and
-        # nothing else is enqueued) -- two extra event records cost ~5 us of stream time per step
+        # nothing else is enqueued) -- two extra event records cost ~5 us of stream time per step.
+        # Also returns the observation rows the caller received from the last step (all ranks' rows at N > 1).
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         inner = gather is not None and gather.mode == "nccl" and not host_io
         kev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)] if inner else ev
+        rows = None
         barrier()
         for k in range(steps):
             flush.fill_(float(k))                            # evict L2 between timed iterations (256 MiB > 126 MB L2)
             ev[k][0].record(stream)
             if host_io:
-                sim.step_host(step0 + k, shared.local if world > 1 else None)
+                rows = sim.step_host(step0 + k, shared.local if world > 1 else None)
                 if world > 1:
                     # N > 1: same call per rank (it returns when this rank's rows are in host memory); shared-memory flags are
                     # the barrier after which the trainer's rank may read every row
                     e2e_step[0] += 1
                     shared.publish_and_wait(e2e_step[0])
+                    rows = shared.all
                 ev[k][1].record(stream)
                 continue
             if inner:
                 kev[k][0].record(stream)
-            obs = sim.step_resident(step0 + k)               # ONE launch: 4 fused sub-steps + observation rows
+            rows = obs = sim.step_resident(step0 + k)        # ONE launch: 4 fused sub-steps + observation rows
             if inner:
                 kev[k][1].record(stream)
             if gather is not None:
-                gather.gather(obs)                           # fused: nothing is enqueued (the launch ends when the rows are complete); nccl mode: the all-gather
+                rows = gather.gather(obs)                    # fused: nothing is enqueued (the launch ends when the rows are complete); nccl mode: the all-gather
             ev[k][1].record(stream)
         barrier()
         ms = sum(a.elapsed_time(b) for a, b in ev)
@@ -462,7 +493,16 @@ def main():
         t = torch.tensor([ms, kms], dtype=torch.float64, device="cuda")
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)         # max over ranks
-        return float(t[0]), float(t[1])
+        return float(t[0]), float(t[1]), rows
+
+    def all_ranks(a):
+        """rows of every rank in rank order (a collective at N > 1: every rank calls it)"""
+        if world == 1:
+            return a
+        t = torch.from_numpy(np.ascontiguousarray(a)).cuda()
+        out = torch.empty((world * t.shape[0],) + tuple(t.shape[1:]), dtype=t.dtype, device="cuda")
+        dist.all_gather_into_tensor(out, t)
+        return out.cpu().numpy()
 
     for k in range(wl.settle):       # workload construction (untimed): land and settle
         control_step(k)
@@ -473,9 +513,17 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_dev, ms_kernel = timed(False, args.steps, W)
+    ms_dev, ms_kernel, rows = timed(False, args.steps, W)
     launches = bt.launch_count() - l0
-    ms_e2e, _ = timed(True, args.steps, W + args.steps)
+    if args.dump_outputs:
+        # read outside the timed region, before the e2e arm advances the state
+        outputs = {"obs": rows.cpu().numpy()}
+        outputs["gc"], outputs["gv"] = (all_ranks(a) for a in bt.get_state())
+    ms_e2e, _, rows = timed(True, args.steps, W + args.steps)
+    if args.dump_outputs:
+        outputs["obs_e2e"] = np.array(rows.numpy() if isinstance(rows, torch.Tensor) else rows)
+        if rank == 0:
+            write_outputs(args.dump_outputs, outputs)
     clocks = sampler.stop() if rank == 0 else None
     st = sim.stats()
     keys = ["mean_contacts_per_env", "mean_solver_sweeps", "non_converged_fraction", "standing_fraction"]
@@ -549,4 +597,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True       # the benchmark leaves the source tree as it found it
     main()

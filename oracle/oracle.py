@@ -7,6 +7,7 @@ algorithms; the RaiSim binary is unavailable, parity with RaiSim itself is unver
 import ctypes as C
 import os
 import subprocess
+import tempfile
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -66,13 +67,15 @@ def _declare(L):
 def lib(which="parity"):
     """parity: liboracle.so, the checker (-ffp-contract=off, portable ISA: bit-stable predicates).
     native: liboracle_native.so, the TIMING build of the same source for bench.py's CPU arm (-O3 -march=native, FMA
-    contraction on), compiled on the machine it is timed on; falls back to the parity build if that fails."""
+    contraction on), compiled on the machine it is timed on into a temporary directory (the source tree may be read-only)
+    and removed once loaded; falls back to the parity build if that fails."""
     if which not in _libs:
         if which == "native":
-            path = os.path.join(_HERE, "liboracle_native.so")
             try:
-                subprocess.check_call(["make", "-C", _HERE, "-s", "-B", "liboracle_native.so"])
-                _libs[which] = _declare(C.CDLL(path))
+                with tempfile.TemporaryDirectory(prefix="oracle_native_") as tmp:
+                    path = os.path.join(tmp, "liboracle_native.so")
+                    subprocess.check_call(["make", "-C", _HERE, "-s", "-B", "native", "NATIVE_LIB=" + path])
+                    _libs[which] = _declare(C.CDLL(path))
             except Exception:
                 _libs[which] = lib("parity")
         else:

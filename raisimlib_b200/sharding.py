@@ -77,7 +77,7 @@ class ObservationGather:
             self.rows = [self._view(mine[0][0]), self._view(mine[1][0])]
             dist.barrier()
         else:
-            self.rows = [torch.empty((world * n, ob_dim), dtype=torch.float32, device="cuda" if torch.cuda.is_available() else "cpu") for _ in range(2)]
+            self.rows = None                                 # allocated by the first gather(), where the rows live (gloo: host)
 
     def _view(self, ptr):
         class _Raw:
@@ -91,6 +91,8 @@ class ObservationGather:
         self.steps += 1
         if self.mode == "peer":
             return self.rows[self.batch.wait_observation_peers()]
+        if self.rows is None:
+            self.rows = [torch.empty((self.world * self.n, self.od), dtype=obs_local.dtype, device=obs_local.device) for _ in range(2)]
         out = self.rows[self.steps & 1]
         allgather_observations(obs_local, out)
         return out

@@ -1101,7 +1101,7 @@ def test_fused_peer_observation_gather_two_gpus(capi):
     NVLink peer memory (CUDA IPC), counters + a wait kernel close the exchange; rows must equal each rank's own rows, in rank order."""
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs two GPUs with peer access")
     import torch.multiprocessing as mp
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
