@@ -234,6 +234,31 @@ class HeightMap {
   std::vector<double> h_;
 };
 
+// World::rayTest() result ([RECALL] upstream RayCollisionList / RayCollisionItem).  Rays see the terrain only (Ground / HeightMap), so a
+// list holds at most one item: the closest hit.  getNormal(), getDistance() and getPairIndex() are extensions of this facade.
+class RayCollisionItem {
+ public:
+  explicit RayCollisionItem(const rsb_ray_hit& h) : h_(h) {}
+  Vec<3> getPosition() const { return {h_.position[0], h_.position[1], h_.position[2]}; }
+  Vec<3> getNormal() const { return {h_.normal[0], h_.normal[1], h_.normal[2]}; }       // unit normal of the triangle hit, +z side
+  double getDistance() const { return h_.distance; }                                       // along the unit direction
+  int getPairIndex() const { return h_.pair_index; }                                       // 0 = Ground, 2*cell+tri on a HeightMap
+  size_t getObjectIndex() const { return 0; }                                              // the terrain is object 0 of the world
+ private:
+  rsb_ray_hit h_;
+};
+class RayCollisionList {
+ public:
+  size_t size() const { return items_.size(); }
+  const RayCollisionItem& operator[](size_t i) const { return items_[i]; }
+  std::vector<RayCollisionItem>::const_iterator begin() const { return items_.begin(); }
+  std::vector<RayCollisionItem>::const_iterator end() const { return items_.end(); }
+  void clear() { items_.clear(); }
+  void push(const rsb_ray_hit& h) { items_.emplace_back(h); }
+ private:
+  std::vector<RayCollisionItem> items_;
+};
+
 // ArticulatedSystem::getSparseJacobian(): the non-zero columns of a 3 x dof Jacobian (the ancestors' dofs only)
 class SparseJacobian {
  public:
@@ -850,6 +875,21 @@ class World {
     int getLoopCounter() const { int32_t it = 0; rsbCheck(rsb_batch_get_solver_iterations(w->w_->batch(), &it, w->env_, 1, RSB_HOST), "getLoopCounter"); return it; }
   };
   ContactSolverView getContactSolver() const { need(); return ContactSolverView{this}; }
+  // upstream World::rayTest: the first crossing of start + t * direction / |direction|, t in [0, length], with this environment's terrain.
+  // The robot is not hit (objectId / localId / mask select among objects upstream; the terrain is the only one here).  Only the closest
+  // hit exists on this path: closestOnly = false is refused.  The terrain is static, so inside a VectorizedEnvironment this costs no
+  // lock-step flush; one launch on the batch's stream and one 32-byte read-back.
+  const RayCollisionList& rayTest(const Vec<3>& start, const Vec<3>& direction, double length, bool closestOnly = true, size_t /*objectId*/ = size_t(-10),
+                                  size_t /*localId*/ = size_t(-10), CollisionGroup /*collisionMask*/ = CollisionGroup(-1)) {
+    if (!closestOnly) throw std::runtime_error("rayTest: only closestOnly = true is implemented (rays see the terrain only: one hit at most)");
+    need();
+    const float o[3] = {float(start[0]), float(start[1]), float(start[2])}, d[3] = {float(direction[0]), float(direction[1]), float(direction[2])};
+    rsb_ray_hit h;
+    rsbCheck(rsb_batch_ray_test(w_->batch(), nullptr, 0, o, d, 1, float(length), &h, env_, 1, RSB_HOST), "rayTest");
+    rays_.clear();
+    if (h.pair_index >= 0) rays_.push(h);
+    return rays_;
+  }
   ArticulatedSystem* getObject(const std::string& name) { return (robot_ && robot_->getName() == name) ? robot_.get() : nullptr; }
   // object-object and self collisions are not part of this path (robot vs terrain only): nothing to ignore
   void ignoreCollisionBetween(size_t, size_t, size_t, size_t) {}
@@ -888,6 +928,7 @@ class World {
   int env_ = 0;
   std::unique_ptr<ArticulatedSystem> robot_;
   Ground ground_; HeightMap hm_;
+  RayCollisionList rays_;
   bool haveGround_ = false;
   double groundZ_ = 0, dt_ = 0.005;
   Vec<3> g_{0, 0, -9.81};

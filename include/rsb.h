@@ -210,6 +210,31 @@ int rsb_batch_observe(rsb_batch* b, float* obs, int env_begin, int env_count, in
  * World::integrate() calls, observation rows out (either pointer may be NULL to skip that leg) */
 int rsb_batch_control_step(rsb_batch* b, const float* ptarget, const float* vtarget, int where_in, int substeps, float* obs, int where_out);
 
+/* ---- terrain sensing (height scans; World::rayTest).  The surface is the one the narrow phase collides with (Ground plane, or each
+ *      environment's height map split into triangles as in DESIGN.md section 2); the robot itself is never hit.  Frame poses describe the
+ *      current state: a frame on body 0 of a floating base is read from the gc rows, any other frame costs one kinematics launch when the
+ *      state changed since the last one.  Pattern arrays (frames, points, frame-fixed rays) are host arrays, uploaded only when they differ
+ *      from the previous call's.  Host outputs are complete on return; device outputs are ordered on the batch's stream. ---- */
+typedef struct rsb_ray_hit {
+  float distance;     /* t of the first crossing, +inf on a miss                                           */
+  float position[3];  /* world-frame hit point (0 on a miss)                                               */
+  float normal[3];    /* unit normal of the triangle hit, oriented +z (terrain -> outside); 0 on a miss    */
+  int32_t pair_index; /* terrain feature: 0 = Ground plane, 2*cell+tri on a HeightMap; -1 = miss           */
+} rsb_ray_hit;        /* 8 words */
+/* out[e * out_stride + f * num_points + k] = z of frame f - terrain height at (p_f + Rz(yaw_f) [x_k, y_k]), yaw_f = atan2(R10, R00) of
+ * the frame's world rotation; points off the map take the height of the nearest border point.  frames[num_frames]
+ * (rsb_model_frame_index) and points_xy[num_points][2] are host arrays; out is `where` memory, out_stride >= num_frames * num_points
+ * (a trainer may write the scan into columns of a wider buffer it owns: the other columns are left as they are). */
+int rsb_batch_height_scan(rsb_batch* b, const int32_t* frames, int num_frames, const float* points_xy, int num_points,
+                          float* out, int out_stride, int env_begin, int env_count, int where);
+/* Rays o + t d/|d|, t in [0, length]: the first crossing of the terrain from either side.
+ * num_frames >= 1: origins / dirs [num_rays][3] (host) are fixed in each frame (rotated with its full world rotation);
+ *                  out [env_count][num_frames][num_rays].
+ * num_frames == 0: origins / dirs [env_count][num_rays][3] are world-frame rays in `where` memory; out [env_count][num_rays].
+ * A zero direction is an error for host arrays; a zero direction read from device memory gives a miss.  No terrain: all misses. */
+int rsb_batch_ray_test(rsb_batch* b, const int32_t* frames, int num_frames, const float* origins, const float* dirs, int num_rays,
+                       float length, rsb_ray_hit* out, int env_begin, int env_count, int where);
+
 /* ---- terrain generation (raisim::TerrainProperties, World::addHeightMap(centerX, centerY, terrainProperties)) ------ */
 typedef struct rsb_terrain_properties {
   int x_samples, y_samples;      /* TerrainProperties::xSamples, ySamples */

@@ -36,6 +36,14 @@ CONTACT_DTYPE = np.dtype([("local_body", np.int32), ("pair_index", np.int32), ("
 assert CONTACT_DTYPE.itemsize == C.sizeof(Contact) == 48
 
 
+class RayHit(C.Structure):
+    _fields_ = [("distance", C.c_float), ("position", C.c_float * 3), ("normal", C.c_float * 3), ("pair_index", C.c_int32)]
+
+
+RAY_HIT_DTYPE = np.dtype([("distance", np.float32), ("position", np.float32, 3), ("normal", np.float32, 3), ("pair_index", np.int32)])
+assert RAY_HIT_DTYPE.itemsize == C.sizeof(RayHit) == 32
+
+
 class ModelTables(C.Structure):
     _fields_ = ([(n, C.c_int) for n in ("nb", "nq", "nv", "floating", "ncoll", "npts")] +
                 [(n, C.POINTER(C.c_int)) for n in ("parent", "jtype", "qidx", "vidx", "depth")] +
@@ -102,7 +110,7 @@ EXPORTED = [
     "rsb_batch_integrate1", "rsb_batch_integrate2", "rsb_batch_integrate",
     "rsb_batch_get_mass_matrix", "rsb_batch_get_nonlinearities", "rsb_batch_get_body_poses", "rsb_batch_get_contacts",
     "rsb_batch_get_contact_points", "rsb_batch_get_solver_iterations", "rsb_batch_get_diverged", "rsb_batch_get_solver_residual", "rsb_batch_get_solver_status", "rsb_batch_update_kinematics", "rsb_batch_device_ptrs", "rsb_batch_launch_count",
-    "rsb_batch_ob_dim", "rsb_batch_observe", "rsb_batch_control_step",
+    "rsb_batch_ob_dim", "rsb_batch_observe", "rsb_batch_control_step", "rsb_batch_height_scan", "rsb_batch_ray_test",
     "rsb_batch_gym_configure", "rsb_batch_gym_reset", "rsb_batch_gym_step",
     "rsb_peer_buffer_create", "rsb_peer_buffer_open", "rsb_peer_buffer_close", "rsb_peer_buffer_destroy", "rsb_batch_set_observation_peers", "rsb_batch_wait_observation_peers",
     "rsb_comm_init", "rsb_comm_allgather_obs", "rsb_comm_destroy", "rsb_terrain_generate", "rsb_heightmap_read_text", "rsb_heightmap_read_png",
@@ -173,6 +181,8 @@ def lib():
         L.rsb_batch_ob_dim.argtypes = [C.c_void_p]
         L.rsb_batch_observe.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
         L.rsb_batch_control_step.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int]
+        L.rsb_batch_height_scan.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]
+        L.rsb_batch_ray_test.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_void_p, C.c_int, C.c_int, C.c_int]
         L.rsb_batch_gym_configure.argtypes = [C.c_void_p] + [C.c_void_p] * 5 + [C.c_int, C.c_float, C.c_float, C.c_float]
         L.rsb_batch_gym_reset.argtypes = [C.c_void_p]
         L.rsb_batch_gym_step.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
@@ -264,6 +274,9 @@ class Model:
 
     def body_index(self, name):
         return _ck(lib().rsb_model_body_index(self.h, name.encode()))
+
+    def frame_index(self, name):
+        return _ck(lib().rsb_model_frame_index(self.h, name.encode()))
 
 
 class Batch:
@@ -522,4 +535,45 @@ class Batch:
             out = np.empty((n, self.ob_dim()), np.float32)
         p, w = _ptr(out)
         _ck(lib().rsb_batch_observe(self.h, p, env_begin, n, w))
+        return out
+
+    # terrain sensing
+    def height_scan(self, frames, points_xy, out=None, out_stride=None, env_begin=0, env_count=None):
+        """p_z - terrain height at the points [P, 2] of each frame's heading frame: out [n, out_stride], columns f * P + k
+        (numpy: host; torch CUDA: device).  frames: frame indices (rsb_model_frame_index) or names."""
+        n = self.n - env_begin if env_count is None else env_count
+        fr = np.ascontiguousarray([self.model.frame_index(f) if isinstance(f, str) else f for f in np.atleast_1d(frames)], np.int32)
+        pts = np.ascontiguousarray(points_xy, np.float32).reshape(-1, 2)
+        width = len(fr) * len(pts)
+        out_stride = width if out_stride is None else out_stride
+        if out is None:
+            out = np.empty((n, out_stride), np.float32)
+        p, w = _ptr(out)
+        _ck(lib().rsb_batch_height_scan(self.h, fr.ctypes.data_as(C.c_void_p), len(fr), pts.ctypes.data_as(C.c_void_p), len(pts), p, out_stride,
+                                        env_begin, n, w))
+        return out
+
+    def ray_test(self, origins, dirs, length, frames=None, out=None, env_begin=0, env_count=None):
+        """first terrain crossing of o + t d/|d|, t in [0, length] -> RAY_HIT_DTYPE records.
+        frames given: origins / dirs [R, 3] fixed in each frame, out [n, F, R].  frames None: world rays [n, R, 3] (numpy or torch CUDA,
+        like out), out [n, R].  A torch CUDA `out` must be a uint8 / int32 / float32 tensor of 32 bytes per record."""
+        n = self.n - env_begin if env_count is None else env_count
+        if frames is not None:
+            fr = np.ascontiguousarray([self.model.frame_index(f) if isinstance(f, str) else f for f in np.atleast_1d(frames)], np.int32)
+            o = np.ascontiguousarray(origins, np.float32).reshape(-1, 3); d = np.ascontiguousarray(dirs, np.float32).reshape(-1, 3)
+            assert o.shape == d.shape
+            nr, shape = len(o), (n, len(fr), len(o))
+            po, pd, pf = o.ctypes.data_as(C.c_void_p), d.ctypes.data_as(C.c_void_p), fr.ctypes.data_as(C.c_void_p)
+            w_in, nf = None, len(fr)
+        else:
+            if not hasattr(origins, "data_ptr"):
+                origins = np.ascontiguousarray(origins, np.float32); dirs = np.ascontiguousarray(dirs, np.float32)
+            assert tuple(origins.shape) == tuple(dirs.shape) and origins.shape[0] == n and origins.shape[-1] == 3
+            (po, w_in), (pd, _) = _ptr(origins), _ptr(dirs)
+            nr, shape, pf, nf = origins.shape[1], (n, origins.shape[1]), None, 0
+        if out is None:
+            out = np.empty(shape, RAY_HIT_DTYPE)
+        p, w = _ptr(out)
+        assert w_in is None or w_in == w, "world rays and the output must both be host or both be device memory"
+        _ck(lib().rsb_batch_ray_test(self.h, pf, nf, po, pd, nr, length, p, env_begin, n, w))
         return out

@@ -14,6 +14,7 @@
 #include "model.hpp"
 #include "step_kernel.cuh"
 #include "aux_kernels.cuh"
+#include "terrain_query.cuh"
 
 using namespace rsb;
 
@@ -83,6 +84,15 @@ struct rsb_batch {
   bool gym_ready = false;
   float *gym_action = nullptr, *gym_obs = nullptr, *gym_reward = nullptr;
   unsigned char* gym_done = nullptr;
+  // terrain sensing (rsb_batch_height_scan / rsb_batch_ray_test)
+  float2* hm_tiles = nullptr;        // per-tile height range of every map, kept beside the map (TqTiles)
+  TqTiles tiles{};
+  float* scan_pat = nullptr;         // device copies of the last height-scan / ray pattern, re-uploaded when the host arrays change
+  float* ray_pat = nullptr;
+  std::vector<float> scan_pat_host, ray_pat_host;
+  size_t scan_pat_cap = 0, ray_pat_cap = 0;
+  float* tq_buf = nullptr;           // world rays in / results bound for host memory
+  size_t tq_buf_bytes = 0;
 };
 
 static int round_up(int x, int m) { return (x + m - 1) / m * m; }
@@ -374,6 +384,26 @@ static int copy_rows_out(rsb_batch* b, float* dst, const float* src, int stride,
   }
   return RSB_OK;
 }
+// coarse grid of the ray test (terrain_query.cuh): [min, max] over the vertices of every TQ_TILE x TQ_TILE-cell tile of every map
+static int build_tiles(rsb_batch* b, int count, int xs, int ys, const float* h) {
+  const int nx = (xs - 1 + TQ_TILE - 1) / TQ_TILE, ny = (ys - 1 + TQ_TILE - 1) / TQ_TILE;
+  std::vector<float2> mm((size_t)count * nx * ny);
+  float lo = h[0], hi = h[0];
+  for (int m = 0; m < count; m++)
+    for (int ty = 0; ty < ny; ty++)
+      for (int tx = 0; tx < nx; tx++) {
+        const float* H = h + (size_t)m * xs * ys;
+        float a = 3.0e38f, c = -3.0e38f;
+        for (int iy = ty * TQ_TILE; iy <= std::min((ty + 1) * TQ_TILE, ys - 1); iy++)
+          for (int ix = tx * TQ_TILE; ix <= std::min((tx + 1) * TQ_TILE, xs - 1); ix++) { a = std::min(a, H[(size_t)iy * xs + ix]); c = std::max(c, H[(size_t)iy * xs + ix]); }
+        mm[((size_t)m * ny + ty) * nx + tx] = make_float2(a, c);
+        lo = std::min(lo, a); hi = std::max(hi, c);
+      }
+  CK(cudaMalloc((void**)&b->hm_tiles, mm.size() * sizeof(float2)));
+  CK(cudaMemcpy(b->hm_tiles, mm.data(), mm.size() * sizeof(float2), cudaMemcpyHostToDevice));
+  b->tiles = TqTiles{b->hm_tiles, nx, ny, lo, hi};
+  return RSB_OK;
+}
 static int check_range(const rsb_batch* b, int env_begin, int env_count) {
   if (!b) return fail(RSB_ERR_INVALID, "null batch");
   if (env_begin < 0 || env_count < 0 || env_begin + env_count > b->N) return fail(RSB_ERR_INVALID, "environment range out of bounds");
@@ -528,7 +558,8 @@ void rsb_batch_destroy(rsb_batch* b) {
   if (b->stream) cudaStreamSynchronize(b->stream);
   for (void* p : {(void*)b->solver_status, (void*)b->resid, (void*)b->diverged, (void*)b->tau_applied, (void*)b->gc, (void*)b->gv, (void*)b->tau, (void*)b->pt, (void*)b->vt, (void*)b->ncontacts, (void*)b->contact_pt, (void*)b->iters,
                   (void*)b->contacts, (void*)b->dbg_M, (void*)b->dbg_h, (void*)b->dbg_R, (void*)b->dbg_p, (void*)b->hmap, (void*)b->staging, (void*)b->obs_staging, (void*)b->blob, (void*)b->gym_const, (void*)b->gym_action,
-                  (void*)b->gym_obs, (void*)b->gym_reward, (void*)b->gym_done, (void*)b->ext, (void*)b->hmap_index, (void*)b->peer_done})
+                  (void*)b->gym_obs, (void*)b->gym_reward, (void*)b->gym_done, (void*)b->ext, (void*)b->hmap_index, (void*)b->peer_done,
+                  (void*)b->hm_tiles, (void*)b->scan_pat, (void*)b->ray_pat, (void*)b->tq_buf})
     if (p) cudaFree(p);
   if (b->own_stream && b->stream) cudaStreamDestroy(b->stream);
   delete b;
@@ -563,9 +594,11 @@ int rsb_batch_set_heightmap(rsb_batch* b, int xs, int ys, float x_size, float y_
   CK(cudaSetDevice(b->device));
   CK(cudaStreamSynchronize(b->stream));
   if (b->hmap) { cudaFree(b->hmap); b->hmap = nullptr; }
+  if (b->hm_tiles) { cudaFree(b->hm_tiles); b->hm_tiles = nullptr; }
   b->ter = TerrainDesc{};               // nothing may point at the freed map if an allocation below fails
   CK(cudaMalloc((void**)&b->hmap, (size_t)xs * ys * 4));
   CK(cudaMemcpy(b->hmap, h, (size_t)xs * ys * 4, cudaMemcpyHostToDevice));
+  int rc = build_tiles(b, 1, xs, ys, h); if (rc) return rc;
   TerrainDesc t{};
   t.type = 2; t.xs = xs; t.ys = ys;
   t.dx = x_size / (float)(xs - 1); t.dy = y_size / (float)(ys - 1); t.inv_dx = 1.0f / t.dx; t.inv_dy = 1.0f / t.dy;
@@ -588,10 +621,12 @@ int rsb_batch_set_heightmaps(rsb_batch* b, int count, int xs, int ys, float x_si
   CK(cudaStreamSynchronize(b->stream));
   if (b->hmap) { cudaFree(b->hmap); b->hmap = nullptr; }
   if (b->hmap_index) { cudaFree(b->hmap_index); b->hmap_index = nullptr; }
+  if (b->hm_tiles) { cudaFree(b->hm_tiles); b->hm_tiles = nullptr; }
   b->ter = TerrainDesc{};               // nothing may point at the freed maps if an allocation below fails
   const size_t words = (size_t)count * xs * ys;
   CK(cudaMalloc((void**)&b->hmap, words * 4));
   CK(cudaMemcpy(b->hmap, h, words * 4, cudaMemcpyHostToDevice));
+  int rc = build_tiles(b, count, xs, ys, h); if (rc) return rc;
   CK(cudaMalloc((void**)&b->hmap_index, (size_t)b->N * 4));
   CK(cudaMemcpy(b->hmap_index, map_of_env, (size_t)b->N * 4, cudaMemcpyHostToDevice));
   TerrainDesc t{};
@@ -927,6 +962,128 @@ int rsb_batch_control_step(rsb_batch* b, const float* ptarget, const float* vtar
     CK(cudaMemcpyAsync(obs, dst, (size_t)b->N * od * 4, cudaMemcpyDeviceToHost, b->stream));
     CK(cudaStreamSynchronize(b->stream));
   } else if (bound_once) CK(cudaStreamSynchronize(b->stream));
+  return RSB_OK;
+}
+
+// ---- terrain sensing: height scans and ray tests (terrain_query.cuh) ----
+// frame records of a pattern (TQ_FRAME_WORDS each); *needs_kin: some frame's pose comes from the getters' pose buffers
+static int pack_frames(const rsb_batch* b, const int32_t* frames, int num_frames, std::vector<float>& pat, bool* needs_kin) {
+  const Model& md = b->model->md;
+  *needs_kin = false;
+  for (int f = 0; f < num_frames; f++) {
+    if (frames[f] < 0 || frames[f] >= (int)md.frames.size()) return fail(RSB_ERR_INVALID, "bad frame index " + std::to_string(frames[f]));
+    const Frame& fr = md.frames[frames[f]];
+    float w[TQ_FRAME_WORDS] = {};
+    std::memcpy(&w[0], &fr.body, 4);
+    for (int k = 0; k < 3; k++) w[1 + k] = (float)fr.pos[k];
+    for (int k = 0; k < 9; k++) w[4 + k] = (float)fr.rot[k];
+    pat.insert(pat.end(), w, w + TQ_FRAME_WORDS);
+    if (fr.body != 0 || !md.floating) *needs_kin = true;
+  }
+  return RSB_OK;
+}
+// device copy of a small host pattern; uploaded only when it differs from the last one (stream order keeps earlier readers safe)
+static int upload_pattern(rsb_batch* b, const std::vector<float>& pat, std::vector<float>& last, float*& dev, size_t& cap) {
+  if (dev && pat.size() == last.size() && std::memcmp(pat.data(), last.data(), pat.size() * 4) == 0) return RSB_OK;
+  if (pat.size() > cap) {
+    if (dev) { CK(cudaStreamSynchronize(b->stream)); cudaFree(dev); dev = nullptr; cap = 0; }
+    last.clear();
+    CK(cudaMalloc((void**)&dev, pat.size() * 4));
+    cap = pat.size();
+  }
+  last.clear();            // a failed copy below must not leave a stale match behind
+  CK(cudaMemcpyAsync(dev, pat.data(), pat.size() * 4, cudaMemcpyHostToDevice, b->stream));
+  last = pat;
+  return RSB_OK;
+}
+static int ensure_tq_buf(rsb_batch* b, size_t bytes) {
+  if (b->tq_buf_bytes >= bytes) return RSB_OK;
+  if (b->tq_buf) { CK(cudaStreamSynchronize(b->stream)); cudaFree(b->tq_buf); b->tq_buf = nullptr; b->tq_buf_bytes = 0; }
+  CK(cudaMalloc((void**)&b->tq_buf, bytes));
+  b->tq_buf_bytes = bytes;
+  return RSB_OK;
+}
+static TqPose tq_pose(const rsb_batch* b) { return TqPose{b->gc, b->gc_stride, b->dbg_R, b->dbg_p, b->nb, b->model->md.floating}; }
+
+int rsb_batch_height_scan(rsb_batch* b, const int32_t* frames, int num_frames, const float* points_xy, int num_points,
+                          float* out, int out_stride, int env_begin, int env_count, int where) {
+  int rc = check_range(b, env_begin, env_count); if (rc) return rc;
+  if (!frames || !points_xy || !out) return fail(RSB_ERR_INVALID, "height scan: null argument");
+  if (num_frames < 1 || num_points < 1) return fail(RSB_ERR_INVALID, "height scan: num_frames and num_points must be >= 1");
+  if ((long long)num_frames * num_points > (1 << 24)) return fail(RSB_ERR_INVALID, "height scan: more than 2^24 samples per environment");
+  if (out_stride < num_frames * num_points) return fail(RSB_ERR_INVALID, "height scan: out_stride " + std::to_string(out_stride) + " < num_frames * num_points = " + std::to_string(num_frames * num_points));
+  if (b->ter.type == 0) return fail(RSB_ERR_INVALID, "height scan: no terrain set (rsb_batch_set_ground / rsb_batch_set_heightmap)");
+  std::vector<float> pat;
+  bool needs_kin = false;
+  rc = pack_frames(b, frames, num_frames, pat, &needs_kin); if (rc) return rc;
+  for (int k = 0; k < 2 * num_points; k++) if (!std::isfinite(points_xy[k])) return fail(RSB_ERR_INVALID, "height scan: non-finite point");
+  if (env_count == 0) return RSB_OK;
+  CK(cudaSetDevice(b->device));
+  pat.insert(pat.end(), points_xy, points_xy + 2 * (size_t)num_points);
+  rc = upload_pattern(b, pat, b->scan_pat_host, b->scan_pat, b->scan_pat_cap); if (rc) return rc;
+  if (needs_kin) { rc = ensure_kinematics(b); if (rc) return rc; }
+  const int per_env = num_frames * num_points;
+  float* dst = out; int stride = out_stride;
+  if (where == RSB_HOST) { rc = ensure_tq_buf(b, (size_t)env_count * per_env * 4); if (rc) return rc; dst = (float*)b->tq_buf; stride = per_env; }
+  const long long total = (long long)env_count * num_frames * ((num_points + TQ_SCAN_PPT - 1) / TQ_SCAN_PPT);
+  rsb_height_scan_kernel<<<(unsigned)((total + 255) / 256), 256, 0, b->stream>>>(b->ter, tq_pose(b), b->scan_pat, num_frames, num_points, env_begin, env_count, dst, stride);
+  CK(cudaGetLastError());
+  b->launches++;
+  if (where == RSB_HOST) {
+    CK(cudaMemcpy2DAsync(out, (size_t)out_stride * 4, dst, (size_t)per_env * 4, (size_t)per_env * 4, env_count, cudaMemcpyDeviceToHost, b->stream));
+    CK(cudaStreamSynchronize(b->stream));
+  }
+  return RSB_OK;
+}
+
+int rsb_batch_ray_test(rsb_batch* b, const int32_t* frames, int num_frames, const float* origins, const float* dirs, int num_rays,
+                       float length, rsb_ray_hit* out, int env_begin, int env_count, int where) {
+  int rc = check_range(b, env_begin, env_count); if (rc) return rc;
+  if (!origins || !dirs || !out || (num_frames > 0 && !frames)) return fail(RSB_ERR_INVALID, "ray test: null argument");
+  if (num_frames < 0 || num_rays < 1) return fail(RSB_ERR_INVALID, "ray test: num_frames must be >= 0 and num_rays >= 1");
+  if ((long long)std::max(num_frames, 1) * num_rays > (1 << 24)) return fail(RSB_ERR_INVALID, "ray test: more than 2^24 rays per environment");
+  if (!(length > 0.f) || !std::isfinite(length)) return fail(RSB_ERR_INVALID, "ray test: length must be finite and > 0");
+  const bool host_rays = num_frames > 0 || where == RSB_HOST;
+  const size_t nray_words = (size_t)3 * num_rays * (num_frames > 0 ? 1 : (size_t)env_count);
+  if (host_rays)
+    for (size_t r = 0; r < nray_words; r += 3) {
+      const double n2 = (double)dirs[r] * dirs[r] + (double)dirs[r + 1] * dirs[r + 1] + (double)dirs[r + 2] * dirs[r + 2];
+      if (!(n2 > 0.0) || !std::isfinite(n2)) return fail(RSB_ERR_INVALID, "ray test: zero or non-finite ray direction");
+    }
+  std::vector<float> pat;
+  bool needs_kin = false;
+  rc = pack_frames(b, frames, num_frames, pat, &needs_kin); if (rc) return rc;
+  if (env_count == 0) return RSB_OK;
+  CK(cudaSetDevice(b->device));
+  const float *org = origins, *dir = dirs;
+  const size_t out_bytes = (size_t)env_count * std::max(num_frames, 1) * num_rays * sizeof(rsb_ray_hit);
+  const size_t in_bytes = (num_frames == 0 && where == RSB_HOST) ? 2 * nray_words * 4 : 0;
+  rc = ensure_tq_buf(b, in_bytes + (where == RSB_HOST ? out_bytes : 0)); if (rc) return rc;
+  if (num_frames > 0) {
+    pat.insert(pat.end(), origins, origins + 3 * (size_t)num_rays);
+    for (int r = 0; r < num_rays; r++) {     // directions are normalised here, in double
+      const double n = std::sqrt((double)dirs[3 * r] * dirs[3 * r] + (double)dirs[3 * r + 1] * dirs[3 * r + 1] + (double)dirs[3 * r + 2] * dirs[3 * r + 2]);
+      for (int k = 0; k < 3; k++) pat.push_back((float)(dirs[3 * r + k] / n));
+    }
+    rc = upload_pattern(b, pat, b->ray_pat_host, b->ray_pat, b->ray_pat_cap); if (rc) return rc;
+    if (needs_kin) { rc = ensure_kinematics(b); if (rc) return rc; }
+    org = dir = nullptr;
+  } else if (where == RSB_HOST) {
+    float* st = (float*)b->tq_buf;
+    CK(cudaMemcpyAsync(st, origins, nray_words * 4, cudaMemcpyHostToDevice, b->stream));
+    CK(cudaMemcpyAsync(st + nray_words, dirs, nray_words * 4, cudaMemcpyHostToDevice, b->stream));
+    org = st; dir = st + nray_words;
+  }
+  rsb_ray_hit* dst = where == RSB_HOST ? reinterpret_cast<rsb_ray_hit*>(reinterpret_cast<char*>(b->tq_buf) + in_bytes) : out;
+  const long long total = (long long)env_count * std::max(num_frames, 1) * num_rays;
+  rsb_ray_test_kernel<<<(unsigned)((total + 255) / 256), 256, 0, b->stream>>>(b->ter, b->tiles, tq_pose(b), b->ray_pat, num_frames, org, dir, num_rays, length,
+                                                                            env_begin, env_count, dst);
+  CK(cudaGetLastError());
+  b->launches++;
+  if (where == RSB_HOST) {
+    CK(cudaMemcpyAsync(out, dst, out_bytes, cudaMemcpyDeviceToHost, b->stream));
+    CK(cudaStreamSynchronize(b->stream));
+  }
   return RSB_OK;
 }
 

@@ -90,6 +90,32 @@ class Batch : public std::enable_shared_from_this<Batch> {
   void control_step(uintptr_t ptarget_dev, int substeps, uintptr_t obs_dev) {
     check(rsb_batch_control_step(b_, reinterpret_cast<const float*>(ptarget_dev), nullptr, RSB_DEVICE, substeps, reinterpret_cast<float*>(obs_dev), RSB_DEVICE), "control_step");
   }
+  void set_heightmap(int xs, int ys, float x_size, float y_size, float cx, float cy, const std::vector<float>& h) {
+    if ((long long)h.size() != (long long)xs * ys) throw std::runtime_error("set_heightmap: need x_samples * y_samples heights");
+    check(rsb_batch_set_heightmap(b_, xs, ys, x_size, y_size, cx, cy, h.data()), "set_heightmap");
+  }
+  // terrain sensing into device memory: out = address of a float32 [env_count, out_stride] tensor (out_stride 0: num_frames * num_points)
+  void height_scan(const std::vector<int32_t>& frames, const std::vector<float>& points_xy, uintptr_t out_dev, int out_stride, int env_begin, int env_count) {
+    if (points_xy.size() % 2) throw std::runtime_error("height_scan: points_xy holds (x, y) pairs");
+    const int np = (int)(points_xy.size() / 2);
+    if (env_count < 0) env_count = view_.num_envs - env_begin;
+    check(rsb_batch_height_scan(b_, frames.data(), (int)frames.size(), points_xy.data(), np, reinterpret_cast<float*>(out_dev),
+                                out_stride > 0 ? out_stride : (int)frames.size() * np, env_begin, env_count, RSB_DEVICE), "height_scan");
+  }
+  // rays fixed in frames (origins / dirs: flat host lists of num_rays * 3); out = address of [env_count, num_frames, num_rays] 32-byte records
+  void ray_test(const std::vector<int32_t>& frames, const std::vector<float>& origins, const std::vector<float>& dirs, float length, uintptr_t out_dev,
+                int env_begin, int env_count) {
+    if (frames.empty() || origins.size() % 3 || dirs.size() != origins.size()) throw std::runtime_error("ray_test: need frames and num_rays * 3 origins and directions");
+    if (env_count < 0) env_count = view_.num_envs - env_begin;
+    check(rsb_batch_ray_test(b_, frames.data(), (int)frames.size(), origins.data(), dirs.data(), (int)(origins.size() / 3), length,
+                             reinterpret_cast<rsb_ray_hit*>(out_dev), env_begin, env_count, RSB_DEVICE), "ray_test");
+  }
+  // world-frame rays from device memory: origins / dirs = addresses of float32 [env_count, num_rays, 3] tensors
+  void ray_test_world(uintptr_t origins_dev, uintptr_t dirs_dev, int num_rays, float length, uintptr_t out_dev, int env_begin, int env_count) {
+    if (env_count < 0) env_count = view_.num_envs - env_begin;
+    check(rsb_batch_ray_test(b_, nullptr, 0, reinterpret_cast<const float*>(origins_dev), reinterpret_cast<const float*>(dirs_dev), num_rays, length,
+                             reinterpret_cast<rsb_ray_hit*>(out_dev), env_begin, env_count, RSB_DEVICE), "ray_test_world");
+  }
   int num_envs() const { return view_.num_envs; }
   int nq() const { return view_.nq; }
   int nv() const { return view_.nv; }
@@ -122,6 +148,14 @@ PYBIND11_MODULE(_rsb_py, m) {
       .def("update_kinematics", &Batch::update_kinematics)
       .def("control_step", &Batch::control_step)
       .def("sync", &Batch::sync)
+      .def("set_heightmap", &Batch::set_heightmap, py::arg("x_samples"), py::arg("y_samples"), py::arg("x_size"), py::arg("y_size"), py::arg("center_x"),
+           py::arg("center_y"), py::arg("heights"))
+      .def("height_scan", &Batch::height_scan, py::arg("frames"), py::arg("points_xy"), py::arg("out"), py::arg("out_stride") = 0, py::arg("env_begin") = 0,
+           py::arg("env_count") = -1, "height scan into a device tensor (address): rsb_batch_height_scan")
+      .def("ray_test", &Batch::ray_test, py::arg("frames"), py::arg("origins"), py::arg("dirs"), py::arg("length"), py::arg("out"), py::arg("env_begin") = 0,
+           py::arg("env_count") = -1, "frame-attached rays into a device buffer of 32-byte records (address): rsb_batch_ray_test")
+      .def("ray_test_world", &Batch::ray_test_world, py::arg("origins"), py::arg("dirs"), py::arg("num_rays"), py::arg("length"), py::arg("out"),
+           py::arg("env_begin") = 0, py::arg("env_count") = -1, "world-frame rays from device tensors (addresses): rsb_batch_ray_test")
       .def_property_readonly("num_envs", &Batch::num_envs)
       .def_property_readonly("nq", &Batch::nq)
       .def_property_readonly("nv", &Batch::nv)
