@@ -75,7 +75,6 @@ def read_heightmap_text(path):
     """World::addHeightMap(raisimHeightMapFileName, ...): -> (heights [ys, xs] float32, x_size, y_size)"""
     xs, ys, sx, sy = C.c_int(), C.c_int(), C.c_double(), C.c_double()
     L = lib()
-    L.rsb_heightmap_read_text.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
     _ck(L.rsb_heightmap_read_text(path.encode(), C.byref(xs), C.byref(ys), C.byref(sx), C.byref(sy), None, 0))
     out = np.empty((ys.value, xs.value), np.float32)
     _ck(L.rsb_heightmap_read_text(path.encode(), C.byref(xs), C.byref(ys), C.byref(sx), C.byref(sy), out.ctypes.data_as(C.c_void_p), out.size))
@@ -86,7 +85,6 @@ def read_heightmap_png(path, height_scale=1.0, height_offset=0.0):
     """World::addHeightMap(pngFileName, cx, cy, xSize, ySize, heightScale, heightOffset): -> heights [ys, xs] float32"""
     xs, ys = C.c_int(), C.c_int()
     L = lib()
-    L.rsb_heightmap_read_png.argtypes = [C.c_char_p, C.c_double, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
     _ck(L.rsb_heightmap_read_png(path.encode(), height_scale, height_offset, C.byref(xs), C.byref(ys), None, 0))
     out = np.empty((ys.value, xs.value), np.float32)
     _ck(L.rsb_heightmap_read_png(path.encode(), height_scale, height_offset, C.byref(xs), C.byref(ys), out.ctypes.data_as(C.c_void_p), out.size))
@@ -135,10 +133,13 @@ def lib():
         L.rsb_model_joint_name.restype = C.c_char_p
         L.rsb_batch_launch_count.restype = C.c_int64
         L.rsb_model_create_from_urdf.argtypes = [C.c_char_p, C.POINTER(C.c_void_p)]
+        L.rsb_model_load.argtypes = [C.c_char_p, C.POINTER(C.c_void_p)]
+        L.rsb_model_save.argtypes = [C.c_void_p, C.c_char_p]
         L.rsb_model_destroy.argtypes = [C.c_void_p]
         L.rsb_model_dims.argtypes = [C.c_void_p] + [C.POINTER(C.c_int)] * 5
         L.rsb_model_get_tables.argtypes = [C.c_void_p, C.POINTER(ModelTables)]
         L.rsb_model_body_index.argtypes = [C.c_void_p, C.c_char_p]
+        L.rsb_model_collision_index.argtypes = [C.c_void_p, C.c_char_p]
         L.rsb_model_body_name.argtypes = [C.c_void_p, C.c_int]
         L.rsb_model_joint_name.argtypes = [C.c_void_p, C.c_int]
         L.rsb_model_frame_index.argtypes = [C.c_void_p, C.c_char_p]
@@ -150,6 +151,7 @@ def lib():
         L.rsb_batch_num_envs.argtypes = [C.c_void_p]
         L.rsb_batch_set_ground.argtypes = [C.c_void_p, C.c_float]
         L.rsb_batch_set_heightmap.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p]
+        L.rsb_batch_set_heightmaps.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_void_p]
         L.rsb_batch_clear_terrain.argtypes = [C.c_void_p]
         L.rsb_batch_set_collision_friction.argtypes = [C.c_void_p, C.c_int, C.c_float]
         L.rsb_batch_set_params.argtypes = [C.c_void_p, C.POINTER(Params)]
@@ -190,6 +192,8 @@ def lib():
         L.rsb_comm_allgather_obs.argtypes = [C.c_void_p, C.POINTER(C.c_void_p)]
         L.rsb_comm_destroy.argtypes = [C.c_void_p]
         L.rsb_terrain_generate.argtypes = [C.POINTER(TerrainProperties), C.c_void_p]
+        L.rsb_heightmap_read_text.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
+        L.rsb_heightmap_read_png.argtypes = [C.c_char_p, C.c_double, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         L.rsb_peer_buffer_create.argtypes = [C.c_int, C.c_size_t, C.POINTER(C.c_void_p), C.c_void_p]
         L.rsb_peer_buffer_open.argtypes = [C.c_int, C.c_void_p, C.POINTER(C.c_void_p)]
         L.rsb_peer_buffer_close.argtypes = [C.c_void_p]
@@ -224,7 +228,6 @@ class Model:
         """URDF path / XML text, or (cache=True) a binary model cache written by Model.save()"""
         h = C.c_void_p()
         if cache:
-            lib().rsb_model_load.argtypes = [C.c_char_p, C.c_void_p]
             _ck(lib().rsb_model_load(path_or_xml.encode(), C.byref(h)))
         else:
             _ck(lib().rsb_model_create_from_urdf(path_or_xml.encode(), C.byref(h)))
@@ -234,11 +237,9 @@ class Model:
         self.nq, self.nv, self.nb, self.ncoll, self.npts = [x.value for x in d]
 
     def collision_index(self, name):
-        lib().rsb_model_collision_index.argtypes = [C.c_void_p, C.c_char_p]
         return _ck(lib().rsb_model_collision_index(self.h, name.encode()))
 
     def save(self, path):
-        lib().rsb_model_save.argtypes = [C.c_void_p, C.c_char_p]
         _ck(lib().rsb_model_save(self.h, path.encode()))
 
     def __del__(self):
@@ -293,6 +294,19 @@ class Batch:
             _lib.rsb_batch_destroy(self.h)
             self.h = None
 
+    def _count(self, env_begin, env_count):
+        """number of environments a call covers: env_count, or every environment from env_begin on when it is None"""
+        return self.n - env_begin if env_count is None else env_count
+
+    def _read(self, getter, row_shape, dtype, env_begin, env_count, range_first=False):
+        """new host array [n, *row_shape] filled by the C getter `getter` for n environments from env_begin.  The getters take
+        (batch, out, env_begin, env_count, where), or with range_first (batch, env_begin, env_count, out, where)."""
+        n = self._count(env_begin, env_count)
+        out = np.empty((n, *row_shape), dtype)
+        p = out.ctypes.data_as(C.c_void_p)
+        _ck(getattr(lib(), getter)(self.h, *((env_begin, n, p) if range_first else (p, env_begin, n)), HOST))
+        return out
+
     # world set-up
     def set_stream(self, stream_ptr):
         _ck(lib().rsb_batch_set_stream(self.h, C.c_void_p(stream_ptr)))
@@ -314,9 +328,7 @@ class Batch:
         count, ys, xs = h.shape
         m = np.ascontiguousarray(map_of_env, np.int32)
         assert m.shape == (self.n,)
-        L = lib()
-        L.rsb_batch_set_heightmaps.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_void_p]
-        _ck(L.rsb_batch_set_heightmaps(self.h, count, xs, ys, x_size, y_size, cx, cy, h.ctypes.data_as(C.c_void_p), m.ctypes.data_as(C.c_void_p)))
+        _ck(lib().rsb_batch_set_heightmaps(self.h, count, xs, ys, x_size, y_size, cx, cy, h.ctypes.data_as(C.c_void_p), m.ctypes.data_as(C.c_void_p)))
 
     def clear_terrain(self):
         _ck(lib().rsb_batch_clear_terrain(self.h))
@@ -340,18 +352,18 @@ class Batch:
 
     # state / actuation
     def set_state(self, gc=None, gv=None, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
+        n = self._count(env_begin, env_count)
         pg, w1 = _ptr(gc); pv, w2 = _ptr(gv)
         _ck(lib().rsb_batch_set_state(self.h, pg, pv, env_begin, n, w1 if gc is not None else w2))
 
     def get_state(self, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
+        n = self._count(env_begin, env_count)
         gc, gv = np.empty((n, self.nq), np.float32), np.empty((n, self.nv), np.float32)
         _ck(lib().rsb_batch_get_state(self.h, gc.ctypes.data_as(C.c_void_p), gv.ctypes.data_as(C.c_void_p), env_begin, n, HOST))
         return gc, gv
 
     def get_state_into(self, gc, gv, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
+        n = self._count(env_begin, env_count)
         pg, w1 = _ptr(gc); pv, w2 = _ptr(gv)
         _ck(lib().rsb_batch_get_state(self.h, pg, pv, env_begin, n, w1 if gc is not None else w2))
 
@@ -361,7 +373,7 @@ class Batch:
         _ck(lib().rsb_batch_set_pd_gains(self.h, kp.ctypes.data_as(C.c_void_p), kd.ctypes.data_as(C.c_void_p)))
 
     def set_pd_target(self, ptarget=None, vtarget=None, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
+        n = self._count(env_begin, env_count)
         pp, w1 = _ptr(ptarget); pv, w2 = _ptr(vtarget)
         _ck(lib().rsb_batch_set_pd_target(self.h, pp, pv, env_begin, n, w1 if ptarget is not None else w2))
 
@@ -374,15 +386,12 @@ class Batch:
         _ck(lib().rsb_batch_bind_pd_target(self.h, C.c_void_p(ptarget_dev.data_ptr()), row_stride or ptarget_dev.shape[-1]))
 
     def set_generalized_force(self, tau, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
+        n = self._count(env_begin, env_count)
         p, w = _ptr(tau)
         _ck(lib().rsb_batch_set_generalized_force(self.h, p, env_begin, n, w))
 
     def generalized_force(self, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
-        out = np.empty((n, self.nv), np.float32)
-        _ck(lib().rsb_batch_get_generalized_force(self.h, out.ctypes.data_as(C.c_void_p), env_begin, n, HOST))
-        return out
+        return self._read("rsb_batch_get_generalized_force", (self.nv,), np.float32, env_begin, env_count)
 
     def set_control_mode(self, mode):
         _ck(lib().rsb_batch_set_control_mode(self.h, mode))
@@ -399,64 +408,43 @@ class Batch:
 
     # read-backs
     def mass_matrix(self, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
-        out = np.empty((n, self.nv, self.nv), np.float32)
-        _ck(lib().rsb_batch_get_mass_matrix(self.h, env_begin, n, out.ctypes.data_as(C.c_void_p), HOST))
-        return out
+        return self._read("rsb_batch_get_mass_matrix", (self.nv, self.nv), np.float32, env_begin, env_count, range_first=True)
 
     def nonlinearities(self, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
-        out = np.empty((n, self.nv), np.float32)
-        _ck(lib().rsb_batch_get_nonlinearities(self.h, env_begin, n, out.ctypes.data_as(C.c_void_p), HOST))
-        return out
+        return self._read("rsb_batch_get_nonlinearities", (self.nv,), np.float32, env_begin, env_count, range_first=True)
 
     def body_poses(self, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
+        n = self._count(env_begin, env_count)
         R, p = np.empty((n, self.nb, 3, 3), np.float32), np.empty((n, self.nb, 3), np.float32)
         _ck(lib().rsb_batch_get_body_poses(self.h, env_begin, n, R.ctypes.data_as(C.c_void_p), p.ctypes.data_as(C.c_void_p), HOST))
         return R, p
 
     def contacts(self, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
+        n = self._count(env_begin, env_count)
         out = np.empty((n, KMAX), CONTACT_DTYPE)
         cnt = np.empty(n, np.int32)
         _ck(lib().rsb_batch_get_contacts(self.h, out.ctypes.data_as(C.c_void_p), cnt.ctypes.data_as(C.c_void_p), env_begin, n, HOST))
         return out, cnt
 
     def contact_points(self, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
-        out = np.empty((n, KMAX), np.int32)
-        _ck(lib().rsb_batch_get_contact_points(self.h, out.ctypes.data_as(C.c_void_p), env_begin, n, HOST))
-        return out
+        return self._read("rsb_batch_get_contact_points", (KMAX,), np.int32, env_begin, env_count)
 
     def solver_iterations(self, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
-        out = np.empty(n, np.int32)
-        _ck(lib().rsb_batch_get_solver_iterations(self.h, out.ctypes.data_as(C.c_void_p), env_begin, n, HOST))
-        return out
+        return self._read("rsb_batch_get_solver_iterations", (), np.int32, env_begin, env_count)
 
     def solver_residual(self, env_begin=0, env_count=None):
         """largest impulse update of the last Gauss-Seidel sweep of every environment (< threshold: converged)"""
-        n = self.n - env_begin if env_count is None else env_count
-        out = np.empty(n, np.float32)
-        _ck(lib().rsb_batch_get_solver_residual(self.h, out.ctypes.data_as(C.c_void_p), env_begin, n, HOST))
-        return out
+        return self._read("rsb_batch_get_solver_residual", (), np.float32, env_begin, env_count)
 
     def solver_status(self, env_begin=0, env_count=None):
         """0 converged, 1 converged on the compliant contact set (stall_reg), 2 stalled, 3 max_iter -- of the last solve"""
-        n = self.n - env_begin if env_count is None else env_count
-        out = np.empty(n, np.int32)
-        _ck(lib().rsb_batch_get_solver_status(self.h, out.ctypes.data_as(C.c_void_p), env_begin, n, HOST))
-        return out
+        return self._read("rsb_batch_get_solver_status", (), np.int32, env_begin, env_count)
 
     def update_kinematics(self):
         _ck(lib().rsb_batch_update_kinematics(self.h))
 
     def diverged(self, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
-        out = np.empty(n, np.int32)
-        _ck(lib().rsb_batch_get_diverged(self.h, out.ctypes.data_as(C.c_void_p), env_begin, n, HOST))
-        return out
+        return self._read("rsb_batch_get_diverged", (), np.int32, env_begin, env_count)
 
     def state_tensors(self):
         """zero-copy torch views of the batch state on its GPU: (gc [N, nq], gv [N, nv]) as strided views of the
@@ -486,7 +474,7 @@ class Batch:
     def set_external_wrench(self, body, force=None, torque=None, point_body=None, env_begin=0, env_count=None):
         """setExternalForce / setExternalTorque: world-frame force / torque rows [n, 3] on `body`, applied at point_body (body
         frame, default = body origin) during the next integrate() / control_step() call only."""
-        n = self.n - env_begin if env_count is None else env_count
+        n = self._count(env_begin, env_count)
         conv = lambda a: a if (a is None or hasattr(a, "data_ptr")) else np.ascontiguousarray(np.broadcast_to(np.asarray(a, np.float32), (n, 3)))
         force, torque = conv(force), conv(torque)
         pf, w1 = _ptr(force); pt_, w2 = _ptr(torque)
@@ -530,7 +518,7 @@ class Batch:
         return par.value
 
     def observe(self, out=None, env_begin=0, env_count=None):
-        n = self.n - env_begin if env_count is None else env_count
+        n = self._count(env_begin, env_count)
         if out is None:
             out = np.empty((n, self.ob_dim()), np.float32)
         p, w = _ptr(out)
@@ -541,7 +529,7 @@ class Batch:
     def height_scan(self, frames, points_xy, out=None, out_stride=None, env_begin=0, env_count=None):
         """p_z - terrain height at the points [P, 2] of each frame's heading frame: out [n, out_stride], columns f * P + k
         (numpy: host; torch CUDA: device).  frames: frame indices (rsb_model_frame_index) or names."""
-        n = self.n - env_begin if env_count is None else env_count
+        n = self._count(env_begin, env_count)
         fr = np.ascontiguousarray([self.model.frame_index(f) if isinstance(f, str) else f for f in np.atleast_1d(frames)], np.int32)
         pts = np.ascontiguousarray(points_xy, np.float32).reshape(-1, 2)
         width = len(fr) * len(pts)
@@ -557,7 +545,7 @@ class Batch:
         """first terrain crossing of o + t d/|d|, t in [0, length] -> RAY_HIT_DTYPE records.
         frames given: origins / dirs [R, 3] fixed in each frame, out [n, F, R].  frames None: world rays [n, R, 3] (numpy or torch CUDA,
         like out), out [n, R].  A torch CUDA `out` must be a uint8 / int32 / float32 tensor of 32 bytes per record."""
-        n = self.n - env_begin if env_count is None else env_count
+        n = self._count(env_begin, env_count)
         if frames is not None:
             fr = np.ascontiguousarray([self.model.frame_index(f) if isinstance(f, str) else f for f in np.atleast_1d(frames)], np.int32)
             o = np.ascontiguousarray(origins, np.float32).reshape(-1, 3); d = np.ascontiguousarray(dirs, np.float32).reshape(-1, 3)

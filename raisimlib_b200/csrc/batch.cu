@@ -62,10 +62,10 @@ struct rsb_batch {
   rsb_contact* contacts = nullptr;
   float *dbg_M = nullptr, *dbg_h = nullptr, *dbg_R = nullptr, *dbg_p = nullptr;
   float* hmap = nullptr;
-  float* staging = nullptr;      // tight-row staging for host<->device repacking
-  float* obs_staging = nullptr;
-  size_t obs_staging_words = 0;
+  float* staging = nullptr;      // tight-row staging for host<->device repacking (staging_slice)
   size_t staging_words = 0, staging_cursor = 0;
+  float* host_out = nullptr;     // results bound for host memory (and world rays in): every user synchronises before it returns
+  size_t host_out_words = 0;
   uint32_t* blob = nullptr;
   std::vector<uint32_t> blob_host;
   BlobHeader hdr{};
@@ -91,8 +91,6 @@ struct rsb_batch {
   float* ray_pat = nullptr;
   std::vector<float> scan_pat_host, ray_pat_host;
   size_t scan_pat_cap = 0, ray_pat_cap = 0;
-  float* tq_buf = nullptr;           // world rays in / results bound for host memory
-  size_t tq_buf_bytes = 0;
 };
 
 static int round_up(int x, int m) { return (x + m - 1) / m * m; }
@@ -210,8 +208,6 @@ static void build_blob(rsb_batch* b) {
   std::memcpy(B.data(), &H, sizeof(H));
 }
 
-static void build_ws_layout(rsb_batch* b) { b->ws = make_ws_layout(b->dims); }
-
 // ------------------------------------------------------------------ launches --------------------
 // static specialisations: every 12-joint quadruped (ANYmal, A1, Go1, ...) shares (13,19,18,floating,3,8);
 // the Atlas-like humanoid is (31,37,36,floating,10,15).  Anything else takes the generic kernel.
@@ -253,7 +249,6 @@ static int pick_config(rsb_batch* b) {
       }
   }
   b->spec = quad_topology ? 1 : (same_dims(b->dims, kHumanoid30) ? 2 : 0);
-  if (const char* e = getenv("RSB_FORCE_GENERIC")) if (atoi(e)) b->spec = 0;
   // Warps per CTA (= resident environments per CTA).  A round of w resident warps per SM costs ~ max(13, w): latency-bound up to a
   // dozen warps (32 k cycles per sub-step), issue-bound beyond (2.5 k cycles per warp; profiles/).  Choose the option with the
   // smallest rounds x cost, ties to the larger CTA (one sub-step barrier group, one copy of
@@ -270,7 +265,6 @@ static int pick_config(rsb_batch* b) {
     const long cost = rounds * std::max(13L, (long)w * ctas);
     if (best == 0 || cost < best_cost) { best = w; best_cost = cost; }
   }
-  if (const char* e = getenv("RSB_FORCE_WPC")) { int w = atoi(e); if (w == 28 || w == 16 || w == 14 || w == 8 || w == 4 || w == 1) if (blob_bytes + (size_t)w * per_warp + 1024 <= budget) best = w; }
   if (best == 0) return fail(RSB_ERR_UNSUPPORTED, "model too large for one warp's shared-memory workspace");
   b->wpc = best;
   b->grid = std::min((b->N + best - 1) / best, best == 14 ? 2 * sms : sms);
@@ -339,13 +333,29 @@ static int do_launch(rsb_batch* b, int substeps, int phase_mask, bool debug, flo
   return RSB_OK;
 }
 
-// rows: tight [n][w] <-> padded [n][stride].  Host buffers go through one CONTIGUOUS PCIe copy into a
-// device staging area and are (un)padded on the device: pitched H2D/D2H copies of 76-byte rows are slow.
-static int ensure_staging(rsb_batch* b, size_t words) {
-  if (b->staging_words >= words) return RSB_OK;
-  if (b->staging) { CK(cudaStreamSynchronize(b->stream)); cudaFree(b->staging); b->staging = nullptr; b->staging_words = 0; }
-  CK(cudaMalloc((void**)&b->staging, words * 4));
-  b->staging_words = words;
+// grows a batch-owned device buffer to at least `count` elements; work already on the stream may still use the old one
+template <class T>
+static int grow(rsb_batch* b, T*& buf, size_t& cap, size_t count) {
+  if (cap >= count) return RSB_OK;
+  if (buf) { CK(cudaStreamSynchronize(b->stream)); cudaFree(buf); buf = nullptr; cap = 0; }
+  CK(cudaMalloc((void**)&buf, count * sizeof(T)));
+  cap = count;
+  return RSB_OK;
+}
+// the next `words` of the staging ring, or null (error recorded).  The ring is reused by back-to-back calls on the same stream:
+// stream order keeps them apart.
+static float* staging_slice(rsb_batch* b, size_t words) {
+  if (grow(b, b->staging, b->staging_words, (size_t)b->N * 64 + 64)) return nullptr;
+  float* st = b->staging + b->staging_cursor;
+  b->staging_cursor = (b->staging_cursor + words + 31) / 32 * 32;
+  if (b->staging_cursor + (size_t)b->N * 40 > b->staging_words) b->staging_cursor = 0;
+  return st;
+}
+// device memory -> the caller's buffer (null: nothing to copy).  RSB_HOST returns with the copy complete; RSB_DEVICE stays
+// stream-ordered.
+static int read_back(rsb_batch* b, void* dst, const void* src, size_t bytes, int where) {
+  if (dst && bytes) CK(cudaMemcpyAsync(dst, src, bytes, where == RSB_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, b->stream));
+  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
   return RSB_OK;
 }
 // device-side alias of a pinned, mapped host allocation (cudaHostAlloc / cudaHostRegister / torch pin_memory); null otherwise
@@ -355,15 +365,14 @@ static const float* mapped_alias(const void* host) {
   if (at.type == cudaMemoryTypeHost && at.devicePointer) return static_cast<const float*>(at.devicePointer);
   return nullptr;
 }
+// rows: tight [n][w] <-> padded [n][stride].  Host buffers go through one CONTIGUOUS PCIe copy into a
+// device staging area and are (un)padded on the device: pitched H2D/D2H copies of 76-byte rows are slow.
 static int copy_rows_in(rsb_batch* b, float* dst, int stride, const float* src, int w, int env_begin, int n, int where) {
   if (!src || n == 0) return RSB_OK;
   const float* dsrc = src;
   if (where == RSB_HOST) {
-    int rc = ensure_staging(b, (size_t)b->N * 64 + 64); if (rc) return rc;
-    // the staging area is reused by back-to-back calls on the same stream: stream order keeps them apart
-    float* st = b->staging + b->staging_cursor;
-    b->staging_cursor = (b->staging_cursor + (size_t)n * w + 31) / 32 * 32;
-    if (b->staging_cursor + (size_t)b->N * 40 > b->staging_words) b->staging_cursor = 0;
+    float* st = staging_slice(b, (size_t)n * w);
+    if (!st) return RSB_ERR_CUDA;
     CK(cudaMemcpyAsync(st, src, (size_t)n * w * 4, cudaMemcpyHostToDevice, b->stream));
     dsrc = st;
   }
@@ -371,18 +380,12 @@ static int copy_rows_in(rsb_batch* b, float* dst, int stride, const float* src, 
   return RSB_OK;
 }
 static int copy_rows_out(rsb_batch* b, float* dst, const float* src, int stride, int w, int env_begin, int n, int where) {
-  if (!dst || n == 0) return RSB_OK;
-  if (where == RSB_HOST) {
-    int rc = ensure_staging(b, (size_t)b->N * 64 + 64); if (rc) return rc;
-    float* st = b->staging + b->staging_cursor;
-    b->staging_cursor = (b->staging_cursor + (size_t)n * w + 31) / 32 * 32;
-    if (b->staging_cursor + (size_t)b->N * 40 > b->staging_words) b->staging_cursor = 0;
-    CK(cudaMemcpy2DAsync(st, (size_t)w * 4, src + (size_t)env_begin * stride, (size_t)stride * 4, (size_t)w * 4, n, cudaMemcpyDeviceToDevice, b->stream));
-    CK(cudaMemcpyAsync(dst, st, (size_t)n * w * 4, cudaMemcpyDeviceToHost, b->stream));
-  } else {
-    CK(cudaMemcpy2DAsync(dst, (size_t)w * 4, src + (size_t)env_begin * stride, (size_t)stride * 4, (size_t)w * 4, n, cudaMemcpyDeviceToDevice, b->stream));
+  float* rows = dst;
+  if (dst && n > 0) {
+    if (where == RSB_HOST && !(rows = staging_slice(b, (size_t)n * w))) return RSB_ERR_CUDA;
+    CK(cudaMemcpy2DAsync(rows, (size_t)w * 4, src + (size_t)env_begin * stride, (size_t)stride * 4, (size_t)w * 4, n, cudaMemcpyDeviceToDevice, b->stream));
   }
-  return RSB_OK;
+  return where == RSB_HOST ? read_back(b, dst, rows, (size_t)n * w * 4, RSB_HOST) : RSB_OK;
 }
 // coarse grid of the ray test (terrain_query.cuh): [min, max] over the vertices of every TQ_TILE x TQ_TILE-cell tile of every map
 static int build_tiles(rsb_batch* b, int count, int xs, int ys, const float* h) {
@@ -403,6 +406,47 @@ static int build_tiles(rsb_batch* b, int count, int xs, int ys, const float* h) 
   CK(cudaMemcpy(b->hm_tiles, mm.data(), mm.size() * sizeof(float2), cudaMemcpyHostToDevice));
   b->tiles = TqTiles{b->hm_tiles, nx, ny, lo, hi};
   return RSB_OK;
+}
+// `count` same-sized height maps back to back and the map of every environment, or (map_of_env null) one map shared by all
+static int install_heightmaps(rsb_batch* b, int count, int xs, int ys, float x_size, float y_size, float cx, float cy, const float* h,
+                              const int32_t* map_of_env) {
+  CK(cudaSetDevice(b->device));
+  CK(cudaStreamSynchronize(b->stream));
+  if (b->hmap) { cudaFree(b->hmap); b->hmap = nullptr; }
+  if (b->hmap_index) { cudaFree(b->hmap_index); b->hmap_index = nullptr; }
+  if (b->hm_tiles) { cudaFree(b->hm_tiles); b->hm_tiles = nullptr; }
+  b->ter = TerrainDesc{};               // nothing may point at the freed maps if an allocation below fails
+  const size_t words = (size_t)count * xs * ys;
+  CK(cudaMalloc((void**)&b->hmap, words * 4));
+  CK(cudaMemcpy(b->hmap, h, words * 4, cudaMemcpyHostToDevice));
+  int rc = build_tiles(b, count, xs, ys, h); if (rc) return rc;
+  TerrainDesc t{};
+  if (map_of_env) {
+    CK(cudaMalloc((void**)&b->hmap_index, (size_t)b->N * 4));
+    CK(cudaMemcpy(b->hmap_index, map_of_env, (size_t)b->N * 4, cudaMemcpyHostToDevice));
+    t.env_map = b->hmap_index; t.map_words = xs * ys;
+  }
+  t.type = 2; t.xs = xs; t.ys = ys;
+  t.dx = x_size / (float)(xs - 1); t.dy = y_size / (float)(ys - 1); t.inv_dx = 1.0f / t.dx; t.inv_dy = 1.0f / t.dy;
+  t.x0 = cx - 0.5f * x_size; t.y0 = cy - 0.5f * y_size;
+  t.xmax = (float)(xs - 1); t.ymax = (float)(ys - 1);
+  t.h = b->hmap;
+  t.hmax = h[0];
+  for (size_t i = 1; i < words; i++) t.hmax = std::max(t.hmax, h[i]);
+  b->ter = t;
+  return RSB_OK;
+}
+// a parsed model, once it fits the kernels (one lane per body, MAX_PT_SLOTS candidate slots per lane); parse errors become RSB_ERR_PARSE
+static int adopt_model(Model (*load)(const std::string&), const char* path, rsb_model** out) {
+  if (!path || !out) return fail(RSB_ERR_INVALID, "null argument");
+  try {
+    std::unique_ptr<rsb_model> m(new rsb_model);      // a parse error thrown below must not leak the half-built model
+    m->md = load(path);
+    if (m->md.nb > 32) return fail(RSB_ERR_UNSUPPORTED, "more than 32 movable bodies (one lane per body)");
+    if (m->md.npts() > 32 * MAX_PT_SLOTS) return fail(RSB_ERR_UNSUPPORTED, "more than 64 candidate contact points");
+    *out = m.release();
+    return RSB_OK;
+  } catch (const std::exception& e) { return fail(RSB_ERR_PARSE, e.what()); }
 }
 static int check_range(const rsb_batch* b, int env_begin, int env_count) {
   if (!b) return fail(RSB_ERR_INVALID, "null batch");
@@ -425,32 +469,12 @@ int rsb_params_default(rsb_params* p) {
 }
 
 // ---- model ---------------------------------------------------------------------------------------
-int rsb_model_create_from_urdf(const char* path_or_xml, rsb_model** out) {
-  if (!path_or_xml || !out) return fail(RSB_ERR_INVALID, "null argument");
-  try {
-    std::unique_ptr<rsb_model> m(new rsb_model);      // a parse error thrown below must not leak the half-built model
-    m->md = load_urdf(path_or_xml);
-    if (m->md.nb > 32) return fail(RSB_ERR_UNSUPPORTED, "more than 32 movable bodies (one lane per body)");
-    if (m->md.npts() > 32 * MAX_PT_SLOTS) return fail(RSB_ERR_UNSUPPORTED, "more than 64 candidate contact points");
-    *out = m.release();
-    return RSB_OK;
-  } catch (const std::exception& e) { return fail(RSB_ERR_PARSE, e.what()); }
-}
+int rsb_model_create_from_urdf(const char* path_or_xml, rsb_model** out) { return adopt_model(load_urdf, path_or_xml, out); }
 int rsb_model_save(const rsb_model* m, const char* path) {
   if (!m || !path) return fail(RSB_ERR_INVALID, "null argument");
   try { save_model(m->md, path); return RSB_OK; } catch (const std::exception& e) { return fail(RSB_ERR_PARSE, e.what()); }
 }
-int rsb_model_load(const char* path, rsb_model** out) {
-  if (!path || !out) return fail(RSB_ERR_INVALID, "null argument");
-  try {
-    std::unique_ptr<rsb_model> m(new rsb_model);
-    m->md = load_model(path);
-    if (m->md.nb > 32) return fail(RSB_ERR_UNSUPPORTED, "more than 32 movable bodies (one lane per body)");
-    if (m->md.npts() > 32 * MAX_PT_SLOTS) return fail(RSB_ERR_UNSUPPORTED, "more than 64 candidate contact points");
-    *out = m.release();
-    return RSB_OK;
-  } catch (const std::exception& e) { return fail(RSB_ERR_PARSE, e.what()); }
-}
+int rsb_model_load(const char* path, rsb_model** out) { return adopt_model(load_model, path, out); }
 void rsb_model_destroy(rsb_model* m) { delete m; }
 int rsb_model_dims(const rsb_model* m, int* nq, int* nv, int* nb, int* ncoll, int* npts) {
   if (!m) return fail(RSB_ERR_INVALID, "null model");
@@ -518,7 +542,7 @@ int rsb_batch_create(const rsb_model* m, int num_envs, int device, rsb_batch** o
   rsb_params_default(&b->prm);
   b->kp.assign(std::max(1, md.nv), 0.f); b->kd.assign(std::max(1, md.nv), 0.f);
   build_blob(b);
-  build_ws_layout(b);
+  b->ws = make_ws_layout(b->dims);
   int rc = pick_config(b);
   if (rc != RSB_OK) { delete b; return rc; }
   size_t N = (size_t)num_envs;
@@ -557,9 +581,9 @@ void rsb_batch_destroy(rsb_batch* b) {
   cudaSetDevice(b->device);
   if (b->stream) cudaStreamSynchronize(b->stream);
   for (void* p : {(void*)b->solver_status, (void*)b->resid, (void*)b->diverged, (void*)b->tau_applied, (void*)b->gc, (void*)b->gv, (void*)b->tau, (void*)b->pt, (void*)b->vt, (void*)b->ncontacts, (void*)b->contact_pt, (void*)b->iters,
-                  (void*)b->contacts, (void*)b->dbg_M, (void*)b->dbg_h, (void*)b->dbg_R, (void*)b->dbg_p, (void*)b->hmap, (void*)b->staging, (void*)b->obs_staging, (void*)b->blob, (void*)b->gym_const, (void*)b->gym_action,
+                  (void*)b->contacts, (void*)b->dbg_M, (void*)b->dbg_h, (void*)b->dbg_R, (void*)b->dbg_p, (void*)b->hmap, (void*)b->staging, (void*)b->host_out, (void*)b->blob, (void*)b->gym_const, (void*)b->gym_action,
                   (void*)b->gym_obs, (void*)b->gym_reward, (void*)b->gym_done, (void*)b->ext, (void*)b->hmap_index, (void*)b->peer_done,
-                  (void*)b->hm_tiles, (void*)b->scan_pat, (void*)b->ray_pat, (void*)b->tq_buf})
+                  (void*)b->hm_tiles, (void*)b->scan_pat, (void*)b->ray_pat})
     if (p) cudaFree(p);
   if (b->own_stream && b->stream) cudaStreamDestroy(b->stream);
   delete b;
@@ -591,24 +615,7 @@ int rsb_batch_clear_terrain(rsb_batch* b) {
 }
 int rsb_batch_set_heightmap(rsb_batch* b, int xs, int ys, float x_size, float y_size, float cx, float cy, const float* h) {
   if (!b || !h || xs < 2 || ys < 2 || !(x_size > 0) || !(y_size > 0)) return fail(RSB_ERR_INVALID, "bad height map");
-  CK(cudaSetDevice(b->device));
-  CK(cudaStreamSynchronize(b->stream));
-  if (b->hmap) { cudaFree(b->hmap); b->hmap = nullptr; }
-  if (b->hm_tiles) { cudaFree(b->hm_tiles); b->hm_tiles = nullptr; }
-  b->ter = TerrainDesc{};               // nothing may point at the freed map if an allocation below fails
-  CK(cudaMalloc((void**)&b->hmap, (size_t)xs * ys * 4));
-  CK(cudaMemcpy(b->hmap, h, (size_t)xs * ys * 4, cudaMemcpyHostToDevice));
-  int rc = build_tiles(b, 1, xs, ys, h); if (rc) return rc;
-  TerrainDesc t{};
-  t.type = 2; t.xs = xs; t.ys = ys;
-  t.dx = x_size / (float)(xs - 1); t.dy = y_size / (float)(ys - 1); t.inv_dx = 1.0f / t.dx; t.inv_dy = 1.0f / t.dy;
-  t.x0 = cx - 0.5f * x_size; t.y0 = cy - 0.5f * y_size;
-  t.xmax = (float)(xs - 1); t.ymax = (float)(ys - 1);
-  t.h = b->hmap;
-  t.hmax = h[0];
-  for (size_t i = 1; i < (size_t)xs * ys; i++) t.hmax = std::max(t.hmax, h[i]);
-  b->ter = t;
-  return RSB_OK;
+  return install_heightmaps(b, 1, xs, ys, x_size, y_size, cx, cy, h, nullptr);
 }
 // terrain atlas (SURVEY 8f N3 "per-env distinct terrains"): `count` same-sized height maps back to back and one map
 // index per environment; every environment collides with its own map, everything else is as rsb_batch_set_heightmap
@@ -617,28 +624,7 @@ int rsb_batch_set_heightmaps(rsb_batch* b, int count, int xs, int ys, float x_si
   if (!b || !h || !map_of_env || count < 1 || xs < 2 || ys < 2 || !(x_size > 0) || !(y_size > 0)) return fail(RSB_ERR_INVALID, "bad height-map atlas");
   if ((size_t)count * xs * ys > ((size_t)1 << 30)) return fail(RSB_ERR_INVALID, "height-map atlas too large");
   for (int e = 0; e < b->N; e++) if (map_of_env[e] < 0 || map_of_env[e] >= count) return fail(RSB_ERR_INVALID, "height-map index out of range");
-  CK(cudaSetDevice(b->device));
-  CK(cudaStreamSynchronize(b->stream));
-  if (b->hmap) { cudaFree(b->hmap); b->hmap = nullptr; }
-  if (b->hmap_index) { cudaFree(b->hmap_index); b->hmap_index = nullptr; }
-  if (b->hm_tiles) { cudaFree(b->hm_tiles); b->hm_tiles = nullptr; }
-  b->ter = TerrainDesc{};               // nothing may point at the freed maps if an allocation below fails
-  const size_t words = (size_t)count * xs * ys;
-  CK(cudaMalloc((void**)&b->hmap, words * 4));
-  CK(cudaMemcpy(b->hmap, h, words * 4, cudaMemcpyHostToDevice));
-  int rc = build_tiles(b, count, xs, ys, h); if (rc) return rc;
-  CK(cudaMalloc((void**)&b->hmap_index, (size_t)b->N * 4));
-  CK(cudaMemcpy(b->hmap_index, map_of_env, (size_t)b->N * 4, cudaMemcpyHostToDevice));
-  TerrainDesc t{};
-  t.type = 2; t.xs = xs; t.ys = ys;
-  t.dx = x_size / (float)(xs - 1); t.dy = y_size / (float)(ys - 1); t.inv_dx = 1.0f / t.dx; t.inv_dy = 1.0f / t.dy;
-  t.x0 = cx - 0.5f * x_size; t.y0 = cy - 0.5f * y_size;
-  t.xmax = (float)(xs - 1); t.ymax = (float)(ys - 1);
-  t.h = b->hmap; t.env_map = b->hmap_index; t.map_words = xs * ys;
-  t.hmax = h[0];
-  for (size_t i = 1; i < words; i++) t.hmax = std::max(t.hmax, h[i]);
-  b->ter = t;
-  return RSB_OK;
+  return install_heightmaps(b, count, xs, ys, x_size, y_size, cx, cy, h, map_of_env);
 }
 int rsb_batch_set_params(rsb_batch* b, const rsb_params* p) {
   if (!b || !p) return fail(RSB_ERR_INVALID, "null argument");
@@ -664,9 +650,7 @@ int rsb_batch_set_state(rsb_batch* b, const float* gc, const float* gv, int env_
 int rsb_batch_get_state(rsb_batch* b, float* gc, float* gv, int env_begin, int env_count, int where) {
   int rc = check_range(b, env_begin, env_count); if (rc) return rc;
   rc = copy_rows_out(b, gc, b->gc, b->gc_stride, b->nq, env_begin, env_count, where); if (rc) return rc;
-  rc = copy_rows_out(b, gv, b->gv, b->gv_stride, b->nv, env_begin, env_count, where); if (rc) return rc;
-  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
-  return RSB_OK;
+  return copy_rows_out(b, gv, b->gv, b->gv_stride, b->nv, env_begin, env_count, where);
 }
 int rsb_batch_set_pd_gains(rsb_batch* b, const float* kp, const float* kd) {
   if (!b || !kp || !kd) return fail(RSB_ERR_INVALID, "null argument");
@@ -712,9 +696,7 @@ int rsb_batch_set_generalized_force(rsb_batch* b, const float* tau, int env_begi
 }
 int rsb_batch_get_generalized_force(rsb_batch* b, float* tau, int env_begin, int env_count, int where) {
   int rc = check_range(b, env_begin, env_count); if (rc) return rc;
-  rc = copy_rows_out(b, tau, b->tau_applied, b->gv_stride, b->nv, env_begin, env_count, where); if (rc) return rc;
-  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
-  return RSB_OK;
+  return copy_rows_out(b, tau, b->tau_applied, b->gv_stride, b->nv, env_begin, env_count, where);
 }
 // ArticulatedSystem::setExternalForce / setExternalTorque for a range of environments: one wrench per environment,
 // acting on `body` at `point_body` (body frame; null = body origin), world-frame force / torque rows (null = zero).
@@ -731,10 +713,8 @@ int rsb_batch_set_external_wrench(rsb_batch* b, int body, const float* force, co
   }
   const float *df = force, *dtq = torque;
   if (where == RSB_HOST && (force || torque)) {
-    rc = ensure_staging(b, (size_t)b->N * 64 + 64); if (rc) return rc;
-    float* st = b->staging + b->staging_cursor;
-    b->staging_cursor = (b->staging_cursor + (size_t)env_count * 6 + 31) / 32 * 32;
-    if (b->staging_cursor + (size_t)b->N * 40 > b->staging_words) b->staging_cursor = 0;
+    float* st = staging_slice(b, (size_t)env_count * 6);
+    if (!st) return RSB_ERR_CUDA;
     if (force) { CK(cudaMemcpyAsync(st, force, (size_t)env_count * 12, cudaMemcpyHostToDevice, b->stream)); df = st; }
     if (torque) { CK(cudaMemcpyAsync(st + (size_t)env_count * 3, torque, (size_t)env_count * 12, cudaMemcpyHostToDevice, b->stream)); dtq = st + (size_t)env_count * 3; }
   }
@@ -795,72 +775,52 @@ int rsb_batch_get_mass_matrix(rsb_batch* b, int env_begin, int env_count, float*
   if (!out) return fail(RSB_ERR_INVALID, "null output buffer");
   if (env_count == 0) return RSB_OK;
   rc = ensure_kinematics(b); if (rc) return rc;
-  size_t w = (size_t)b->nv * b->nv;
-  CK(cudaMemcpyAsync(out, b->dbg_M + env_begin * w, env_count * w * 4, where == RSB_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, b->stream));
-  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
-  return RSB_OK;
+  const size_t w = (size_t)b->nv * b->nv;
+  return read_back(b, out, b->dbg_M + env_begin * w, env_count * w * 4, where);
 }
 int rsb_batch_get_nonlinearities(rsb_batch* b, int env_begin, int env_count, float* out, int where) {
   int rc = check_range(b, env_begin, env_count); if (rc) return rc;
   if (!out) return fail(RSB_ERR_INVALID, "null output buffer");
   if (env_count == 0) return RSB_OK;
   rc = ensure_kinematics(b); if (rc) return rc;
-  CK(cudaMemcpyAsync(out, b->dbg_h + (size_t)env_begin * b->nv, (size_t)env_count * b->nv * 4, where == RSB_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, b->stream));
-  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
-  return RSB_OK;
+  return read_back(b, out, b->dbg_h + (size_t)env_begin * b->nv, (size_t)env_count * b->nv * 4, where);
 }
 int rsb_batch_get_body_poses(rsb_batch* b, int env_begin, int env_count, float* rot, float* pos, int where) {
   int rc = check_range(b, env_begin, env_count); if (rc) return rc;
   if (env_count == 0) return RSB_OK;
   rc = ensure_kinematics(b); if (rc) return rc;
-  cudaMemcpyKind kind = where == RSB_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-  if (rot) CK(cudaMemcpyAsync(rot, b->dbg_R + (size_t)env_begin * b->nb * 9, (size_t)env_count * b->nb * 9 * 4, kind, b->stream));
-  if (pos) CK(cudaMemcpyAsync(pos, b->dbg_p + (size_t)env_begin * b->nb * 3, (size_t)env_count * b->nb * 3 * 4, kind, b->stream));
-  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
-  return RSB_OK;
+  rc = read_back(b, rot, b->dbg_R + (size_t)env_begin * b->nb * 9, (size_t)env_count * b->nb * 9 * 4, where); if (rc) return rc;
+  return read_back(b, pos, b->dbg_p + (size_t)env_begin * b->nb * 3, (size_t)env_count * b->nb * 3 * 4, where);
 }
 int rsb_batch_get_contacts(rsb_batch* b, rsb_contact* out, int32_t* counts, int env_begin, int env_count, int where) {
   int rc = check_range(b, env_begin, env_count); if (rc) return rc;
-  cudaMemcpyKind kind = where == RSB_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-  if (out) CK(cudaMemcpyAsync(out, b->contacts + (size_t)env_begin * KMAX, (size_t)env_count * KMAX * sizeof(rsb_contact), kind, b->stream));
-  if (counts) CK(cudaMemcpyAsync(counts, b->ncontacts + env_begin, (size_t)env_count * 4, kind, b->stream));
-  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
-  return RSB_OK;
+  rc = read_back(b, out, b->contacts + (size_t)env_begin * KMAX, (size_t)env_count * KMAX * sizeof(rsb_contact), where); if (rc) return rc;
+  return read_back(b, counts, b->ncontacts + env_begin, (size_t)env_count * 4, where);
 }
 int rsb_batch_get_contact_points(rsb_batch* b, int32_t* pt, int env_begin, int env_count, int where) {
   int rc = check_range(b, env_begin, env_count); if (rc) return rc;
   if (!pt) return fail(RSB_ERR_INVALID, "null output buffer");
-  CK(cudaMemcpyAsync(pt, b->contact_pt + (size_t)env_begin * KMAX, (size_t)env_count * KMAX * 4, where == RSB_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, b->stream));
-  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
-  return RSB_OK;
+  return read_back(b, pt, b->contact_pt + (size_t)env_begin * KMAX, (size_t)env_count * KMAX * 4, where);
 }
 int rsb_batch_get_solver_iterations(rsb_batch* b, int32_t* it, int env_begin, int env_count, int where) {
   int rc = check_range(b, env_begin, env_count); if (rc) return rc;
   if (!it) return fail(RSB_ERR_INVALID, "null output buffer");
-  CK(cudaMemcpyAsync(it, b->iters + env_begin, (size_t)env_count * 4, where == RSB_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, b->stream));
-  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
-  return RSB_OK;
+  return read_back(b, it, b->iters + env_begin, (size_t)env_count * 4, where);
 }
 int rsb_batch_get_solver_status(rsb_batch* b, int32_t* status, int env_begin, int env_count, int where) {
   int rc = check_range(b, env_begin, env_count); if (rc) return rc;
   if (!status) return fail(RSB_ERR_INVALID, "null output buffer");
-  CK(cudaMemcpyAsync(status, b->solver_status + env_begin, (size_t)env_count * 4, where == RSB_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, b->stream));
-  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
-  return RSB_OK;
+  return read_back(b, status, b->solver_status + env_begin, (size_t)env_count * 4, where);
 }
 int rsb_batch_get_solver_residual(rsb_batch* b, float* resid, int env_begin, int env_count, int where) {
   int rc = check_range(b, env_begin, env_count); if (rc) return rc;
   if (!resid) return fail(RSB_ERR_INVALID, "null output buffer");
-  CK(cudaMemcpyAsync(resid, b->resid + env_begin, (size_t)env_count * 4, where == RSB_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, b->stream));
-  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
-  return RSB_OK;
+  return read_back(b, resid, b->resid + env_begin, (size_t)env_count * 4, where);
 }
 int rsb_batch_get_diverged(rsb_batch* b, int32_t* flags, int env_begin, int env_count, int where) {
   int rc = check_range(b, env_begin, env_count); if (rc) return rc;
   if (!flags) return fail(RSB_ERR_INVALID, "null output buffer");
-  CK(cudaMemcpyAsync(flags, b->diverged + env_begin, (size_t)env_count * 4, where == RSB_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, b->stream));
-  if (where == RSB_HOST) CK(cudaStreamSynchronize(b->stream));
-  return RSB_OK;
+  return read_back(b, flags, b->diverged + env_begin, (size_t)env_count * 4, where);
 }
 int rsb_batch_device_ptrs(rsb_batch* b, rsb_device_view* v) {
   if (!b || !v) return fail(RSB_ERR_INVALID, "null argument");
@@ -875,36 +835,26 @@ int rsb_batch_ob_dim(const rsb_batch* b) {
   if (!b) return 0;
   return b->model->md.floating ? (b->nq + b->nv - 3) : (b->nq + b->nv);
 }
-static int observe_impl(rsb_batch* b, float* obs, int env_begin, int env_count, int where, bool sync) {
+static int observe_impl(rsb_batch* b, float* obs, int env_begin, int env_count, int where) {
   const int od = rsb_batch_ob_dim(b);
   float* dst = obs;
   if (where == RSB_HOST) {
-    size_t need = (size_t)b->N * od;
-    if (b->obs_staging_words < need) {
-      if (b->obs_staging) { CK(cudaStreamSynchronize(b->stream)); cudaFree(b->obs_staging); }
-      b->obs_staging = nullptr; b->obs_staging_words = 0;
-      CK(cudaMalloc((void**)&b->obs_staging, need * 4));
-      b->obs_staging_words = need;
-    }
-    dst = b->obs_staging;
+    int rc = grow(b, b->host_out, b->host_out_words, (size_t)b->N * od); if (rc) return rc;
+    dst = b->host_out;
   }
   int threads = 128, blocks = (env_count * 32 + threads - 1) / threads;
   rsb_observe_kernel<<<blocks, threads, 0, b->stream>>>(b->gc + (size_t)env_begin * b->gc_stride, b->gv + (size_t)env_begin * b->gv_stride,
                                                          b->gc_stride, b->gv_stride, b->nq, b->nv, b->model->md.floating, env_count, dst, od);
   CK(cudaGetLastError());
   b->launches++;
-  if (where == RSB_HOST) {
-    CK(cudaMemcpyAsync(obs, dst, (size_t)env_count * od * 4, cudaMemcpyDeviceToHost, b->stream));
-    if (sync) CK(cudaStreamSynchronize(b->stream));
-  }
-  return RSB_OK;
+  return where == RSB_HOST ? read_back(b, obs, dst, (size_t)env_count * od * 4, RSB_HOST) : RSB_OK;
 }
 int rsb_batch_observe(rsb_batch* b, float* obs, int env_begin, int env_count, int where) {
   int rc = check_range(b, env_begin, env_count); if (rc) return rc;
   if (!obs) return fail(RSB_ERR_INVALID, "null obs");
   if (env_count == 0) return RSB_OK;
   CK(cudaSetDevice(b->device));
-  return observe_impl(b, obs, env_begin, env_count, where, true);
+  return observe_impl(b, obs, env_begin, env_count, where);
 }
 
 // VectorizedEnvironment::step() for the whole batch in ONE call: PD targets in, `substeps` fused
@@ -934,34 +884,22 @@ int rsb_batch_control_step(rsb_batch* b, const float* ptarget, const float* vtar
   const bool bound_once = b->pt_once || b->vt_once;
   if (!obs || !b->model->md.floating) {
     rc = do_launch(b, substeps, 0, false); if (rc) return rc;
-    if (obs) rc = observe_impl(b, obs, 0, b->N, where_out, true);
+    if (obs) rc = observe_impl(b, obs, 0, b->N, where_out);
     if (bound_once) CK(cudaStreamSynchronize(b->stream));   // the caller may reuse its pinned target buffer on return
     return rc;
   }
-  // observation rows are written by the step kernel itself (no separate observe launch)
-  float* dst = obs;
-  const int od = rsb_batch_ob_dim(b);
-  float* obs_alias = where_out == RSB_HOST ? const_cast<float*>(mapped_alias(obs)) : nullptr;
-  if (obs_alias) {   // observation rows go straight to the caller's pinned buffer as each environment finishes
-    rc = do_launch(b, substeps, 0, false, obs_alias); if (rc) return rc;
-    CK(cudaStreamSynchronize(b->stream));
-    return RSB_OK;
-  }
-  if (where_out == RSB_HOST) {
-    size_t need = (size_t)b->N * od;
-    if (b->obs_staging_words < need) {
-      if (b->obs_staging) { CK(cudaStreamSynchronize(b->stream)); cudaFree(b->obs_staging); }
-      b->obs_staging = nullptr; b->obs_staging_words = 0;
-      CK(cudaMalloc((void**)&b->obs_staging, need * 4));
-      b->obs_staging_words = need;
-    }
-    dst = b->obs_staging;
+  // observation rows are written by the step kernel itself (no separate observe launch): into the caller's device rows, straight
+  // into its pinned host buffer as each environment finishes, or (pageable host memory) into host_out and then one copy
+  float* dst = where_out == RSB_HOST ? const_cast<float*>(mapped_alias(obs)) : obs;
+  const bool staged = !dst;
+  const size_t obs_words = (size_t)b->N * rsb_batch_ob_dim(b);
+  if (staged) {
+    rc = grow(b, b->host_out, b->host_out_words, obs_words); if (rc) return rc;
+    dst = b->host_out;
   }
   rc = do_launch(b, substeps, 0, false, dst, where_out == RSB_DEVICE); if (rc) return rc;
-  if (where_out == RSB_HOST) {
-    CK(cudaMemcpyAsync(obs, dst, (size_t)b->N * od * 4, cudaMemcpyDeviceToHost, b->stream));
-    CK(cudaStreamSynchronize(b->stream));
-  } else if (bound_once) CK(cudaStreamSynchronize(b->stream));
+  if (staged) return read_back(b, obs, dst, obs_words * 4, RSB_HOST);
+  if (where_out == RSB_HOST || bound_once) CK(cudaStreamSynchronize(b->stream));
   return RSB_OK;
 }
 
@@ -985,22 +923,10 @@ static int pack_frames(const rsb_batch* b, const int32_t* frames, int num_frames
 // device copy of a small host pattern; uploaded only when it differs from the last one (stream order keeps earlier readers safe)
 static int upload_pattern(rsb_batch* b, const std::vector<float>& pat, std::vector<float>& last, float*& dev, size_t& cap) {
   if (dev && pat.size() == last.size() && std::memcmp(pat.data(), last.data(), pat.size() * 4) == 0) return RSB_OK;
-  if (pat.size() > cap) {
-    if (dev) { CK(cudaStreamSynchronize(b->stream)); cudaFree(dev); dev = nullptr; cap = 0; }
-    last.clear();
-    CK(cudaMalloc((void**)&dev, pat.size() * 4));
-    cap = pat.size();
-  }
-  last.clear();            // a failed copy below must not leave a stale match behind
+  last.clear();            // a failed allocation or copy below must not leave a stale match behind
+  int rc = grow(b, dev, cap, pat.size()); if (rc) return rc;
   CK(cudaMemcpyAsync(dev, pat.data(), pat.size() * 4, cudaMemcpyHostToDevice, b->stream));
   last = pat;
-  return RSB_OK;
-}
-static int ensure_tq_buf(rsb_batch* b, size_t bytes) {
-  if (b->tq_buf_bytes >= bytes) return RSB_OK;
-  if (b->tq_buf) { CK(cudaStreamSynchronize(b->stream)); cudaFree(b->tq_buf); b->tq_buf = nullptr; b->tq_buf_bytes = 0; }
-  CK(cudaMalloc((void**)&b->tq_buf, bytes));
-  b->tq_buf_bytes = bytes;
   return RSB_OK;
 }
 static TqPose tq_pose(const rsb_batch* b) { return TqPose{b->gc, b->gc_stride, b->dbg_R, b->dbg_p, b->nb, b->model->md.floating}; }
@@ -1024,7 +950,7 @@ int rsb_batch_height_scan(rsb_batch* b, const int32_t* frames, int num_frames, c
   if (needs_kin) { rc = ensure_kinematics(b); if (rc) return rc; }
   const int per_env = num_frames * num_points;
   float* dst = out; int stride = out_stride;
-  if (where == RSB_HOST) { rc = ensure_tq_buf(b, (size_t)env_count * per_env * 4); if (rc) return rc; dst = (float*)b->tq_buf; stride = per_env; }
+  if (where == RSB_HOST) { rc = grow(b, b->host_out, b->host_out_words, (size_t)env_count * per_env); if (rc) return rc; dst = b->host_out; stride = per_env; }
   const long long total = (long long)env_count * num_frames * ((num_points + TQ_SCAN_PPT - 1) / TQ_SCAN_PPT);
   rsb_height_scan_kernel<<<(unsigned)((total + 255) / 256), 256, 0, b->stream>>>(b->ter, tq_pose(b), b->scan_pat, num_frames, num_points, env_begin, env_count, dst, stride);
   CK(cudaGetLastError());
@@ -1057,8 +983,8 @@ int rsb_batch_ray_test(rsb_batch* b, const int32_t* frames, int num_frames, cons
   CK(cudaSetDevice(b->device));
   const float *org = origins, *dir = dirs;
   const size_t out_bytes = (size_t)env_count * std::max(num_frames, 1) * num_rays * sizeof(rsb_ray_hit);
-  const size_t in_bytes = (num_frames == 0 && where == RSB_HOST) ? 2 * nray_words * 4 : 0;
-  rc = ensure_tq_buf(b, in_bytes + (where == RSB_HOST ? out_bytes : 0)); if (rc) return rc;
+  const size_t in_words = (num_frames == 0 && where == RSB_HOST) ? 2 * nray_words : 0;
+  rc = grow(b, b->host_out, b->host_out_words, in_words + (where == RSB_HOST ? out_bytes / 4 : 0)); if (rc) return rc;
   if (num_frames > 0) {
     pat.insert(pat.end(), origins, origins + 3 * (size_t)num_rays);
     for (int r = 0; r < num_rays; r++) {     // directions are normalised here, in double
@@ -1069,22 +995,18 @@ int rsb_batch_ray_test(rsb_batch* b, const int32_t* frames, int num_frames, cons
     if (needs_kin) { rc = ensure_kinematics(b); if (rc) return rc; }
     org = dir = nullptr;
   } else if (where == RSB_HOST) {
-    float* st = (float*)b->tq_buf;
+    float* st = b->host_out;
     CK(cudaMemcpyAsync(st, origins, nray_words * 4, cudaMemcpyHostToDevice, b->stream));
     CK(cudaMemcpyAsync(st + nray_words, dirs, nray_words * 4, cudaMemcpyHostToDevice, b->stream));
     org = st; dir = st + nray_words;
   }
-  rsb_ray_hit* dst = where == RSB_HOST ? reinterpret_cast<rsb_ray_hit*>(reinterpret_cast<char*>(b->tq_buf) + in_bytes) : out;
+  rsb_ray_hit* dst = where == RSB_HOST ? reinterpret_cast<rsb_ray_hit*>(b->host_out + in_words) : out;
   const long long total = (long long)env_count * std::max(num_frames, 1) * num_rays;
   rsb_ray_test_kernel<<<(unsigned)((total + 255) / 256), 256, 0, b->stream>>>(b->ter, b->tiles, tq_pose(b), b->ray_pat, num_frames, org, dir, num_rays, length,
                                                                             env_begin, env_count, dst);
   CK(cudaGetLastError());
   b->launches++;
-  if (where == RSB_HOST) {
-    CK(cudaMemcpyAsync(out, dst, out_bytes, cudaMemcpyDeviceToHost, b->stream));
-    CK(cudaStreamSynchronize(b->stream));
-  }
-  return RSB_OK;
+  return where == RSB_HOST ? read_back(b, out, dst, out_bytes, RSB_HOST) : RSB_OK;
 }
 
 // ---- RaisimGym ANYmal task (SURVEY 8f N1): VectorizedEnvironment::{reset, step, observe} for the whole batch ----
@@ -1210,10 +1132,11 @@ int rsb_batch_set_observation_peers(rsb_batch* b, int world, int rank, void* con
   for (int p = 0; p < world; p++) if (!obs_all[2 * p] || !obs_all[2 * p + 1] || !flags[p]) return fail(RSB_ERR_INVALID, "null peer buffer");
   CK(cudaSetDevice(b->device));
   CK(cudaStreamSynchronize(b->stream));
-  for (int p = 0; p < world; p++) { b->peer_obs[p][0] = (float*)obs_all[2 * p]; b->peer_obs[p][1] = (float*)obs_all[2 * p + 1]; b->peer_flag[p] = (unsigned*)flags[p]; }
-  b->peer_world = world; b->peer_rank = rank; b->peer_epoch = 0;
+  b->peer_world = 0;                    // a failure below leaves the gather off
   if (!b->peer_done) CK(cudaMalloc(&b->peer_done, sizeof(unsigned)));
   CK(cudaMemsetAsync(b->peer_done, 0, sizeof(unsigned), b->stream));
+  for (int p = 0; p < world; p++) { b->peer_obs[p][0] = (float*)obs_all[2 * p]; b->peer_obs[p][1] = (float*)obs_all[2 * p + 1]; b->peer_flag[p] = (unsigned*)flags[p]; }
+  b->peer_world = world; b->peer_rank = rank; b->peer_epoch = 0;
   return RSB_OK;
 }
 // *buffer_parity (optional) = which of this rank's two buffers holds the rows of the LAST control step of every rank.  The arrival
@@ -1221,12 +1144,6 @@ int rsb_batch_set_observation_peers(rsb_batch* b, int world, int rank, void* con
 // after the step the rows are complete and nothing is enqueued here.
 int rsb_batch_wait_observation_peers(rsb_batch* b, int* buffer_parity) {
   if (!b || b->peer_world <= 0 || b->peer_epoch == 0) return fail(RSB_ERR_INVALID, "no fused observation gather in flight");
-  if (!b->peer_done) {       // (unreachable with rsb_batch_set_observation_peers; kept as the stand-alone form of the wait)
-    CK(cudaSetDevice(b->device));
-    rsb_peer_wait_kernel<<<1, 32, 0, b->stream>>>(b->peer_flag[b->peer_rank], b->peer_world, b->peer_epoch * (unsigned)b->grid, 20000000000ll /* ~10 s of SM clocks */);
-    CK(cudaGetLastError());
-    b->launches++;
-  }
   if (buffer_parity) *buffer_parity = (int)((b->peer_epoch - 1) & 1);
   return RSB_OK;
 }

@@ -206,7 +206,7 @@ struct StepArgs {
   unsigned* peer_flag[MAX_PEERS];  // peer p's arrival counters [world]: += 1 per finished CTA of this rank
   int peer_world, peer_rank;
   unsigned peer_expected;          // arrival count every rank's counter reaches when its rows of THIS step have landed (steps so far x CTAs)
-  unsigned* peer_done;             // CTAs of this launch that finished: the last one waits for the peers (null: the caller enqueues rsb_peer_wait_kernel)
+  unsigned* peer_done;             // CTAs of this launch that finished: the last one waits for the peers (set whenever peer_world > 0)
   // RaisimGym task fused into the step (rsb_batch_gym_step): the launch turns the action rows into PD targets before the first
   // sub-step and, after the last one, computes reward and termination, resets the terminated environments and writes the
   // observation rows of the (possibly reset) state -- VectorizedEnvironment::step() + observe() in ONE launch
@@ -1534,20 +1534,6 @@ __global__ void __launch_bounds__(WPC * 32, (WPC == 14 ? 2 : 1)) rsb_step_kernel
         }
       }
     }
-  }
-}
-
-// Arrival wait of the fused observation all-gather: lane r returns when rank r's `expected` CTAs have signalled, i.e. when every
-// row of that rank's step has landed in THIS GPU's gathered buffer.  Bounded: a dead peer traps instead of hanging the GPU.
-__global__ void rsb_peer_wait_kernel(const unsigned* flags, int world, unsigned expected, long long max_cycles) {
-  if ((int)threadIdx.x >= world) return;
-  const volatile unsigned* f = flags + threadIdx.x;
-  const long long t0 = clock64();
-  for (;;) {
-    unsigned v;
-    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(f) : "memory");
-    if ((int)(v - expected) >= 0) break;
-    if (clock64() - t0 > max_cycles) __trap();
   }
 }
 
